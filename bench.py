@@ -4,6 +4,7 @@ bench.py -- NLMeansFilter throughput on B200, one JSON line (driver contract).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                   [--workload cfg3|cfg2|cfg1|cfg4|cfg5] [--rows R] [--semantics as_written|reference_compiled]
+                  [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
   python bench.py --apply-njobs N      single process: NLMeansFilter(...).apply(ds, njobs=N) on a host Dataset
 
@@ -31,6 +32,11 @@ kernels + D2H inside the timed region), with the copy-only ceiling of the same p
 `parity` compares sampled sub-cubes of the benchmarked cube (true corner, slab / rank seam, interior) with the oracle
 (C restatement pinned bit-exact to the compiled reference) in the same run; above 1e-4 the run fails.
 `cpu_baseline` times the reference's own Cython kernel on the host cores on a bounded crop.
+
+--dump-outputs DIR writes what the last timed step computed, the (rows, nx, nt, V) float32 result of each rank, as
+DIR/out.npy (DIR/out_rank<k>.npy for N > 1): a (K, V) array of K voxels in memory order, every voxel when the result
+fits in 48 MB / N, else a fixed seeded sample (`dump_sample`).  The inputs depend on the arguments only, so two builds
+of the project can be compared output for output.
 """
 import argparse
 import json
@@ -65,10 +71,23 @@ WORKLOADS = {
 METRIC = "NLMeansFilter Mvoxel/s"
 UNIT = "Mvoxel/s"
 PARITY_TOL = 1e-4
+DUMP_BYTES = 48 << 20          # --dump-outputs: all ranks together
 
 
 def fvec(wl):
     return tuple(wl["f"] if x > 0 else 0 for x in wl["r"])
+
+
+def dump_sample(shape, world, seed=1234):
+    """(y, x, t) coordinates of the voxels --dump-outputs writes of a (ny, nx, nt, V) float32 result, in memory order:
+    every voxel when the result fits in DUMP_BYTES / world, else a seeded sample of that many voxels."""
+    import numpy as np
+    ny, nx, nt, V = shape
+    n, k = ny * nx * nt, DUMP_BYTES // world // (4 * V)
+    flat = np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+    y, rest = np.divmod(flat, nx * nt)
+    x, t = np.divmod(rest, nt)
+    return y, x, t
 
 
 def peaks():
@@ -420,6 +439,11 @@ def run_ours(args):
         seams.append(("rank_seam", ny - 1))
     samples = parity_samples(wl, ny, global_rows, world, seams) if rank == 0 else []
     blocks = [None] * len(samples)
+    dump = None                    # --dump-outputs: the sampled voxels and, once the last timed step ran, their values
+    if args.dump_outputs:
+        ys, xs, ts = dump_sample((ny, nx, nt, V), world)
+        dump = {"y": ys, "idx": [torch.from_numpy(a).to(dev) for a in (ys, xs, ts)], "last_step": False,
+                "values": torch.empty((len(ys), V), dtype=torch.float32, device=dev) if streamed else None}
 
     kev = []                       # CUDA events around every nlm kernel launch of the timed region
     plan_info = {}
@@ -472,6 +496,10 @@ def run_ours(args):
                         blocks[i] = torch.zeros((s["y"][1] - s["y"][0], s["x"][1] - s["x"][0], s["t"][1] - s["t"][0], V),
                                                 dtype=torch.float32, device=dev)
                     blocks[i][a - s["y"][0]:b - s["y"][0]] = res[a - lo:b - lo, s["x"][0]:s["x"][1], s["t"][0]:s["t"][1]]
+            if dump is not None and dump["last_step"]:          # the slabs are not kept: gather while they pass
+                a, b = np.searchsorted(dump["y"], (lo, hi))
+                y, x, t = (i[a:b] for i in dump["idx"])
+                dump["values"][a:b] = res[y - lo, x, t]
 
         def on_kernel(before, plan):
             state["plan"] = plan
@@ -518,6 +546,8 @@ def run_ours(args):
     barrier()
     e0.record()
     for i in range(args.steps):
+        if dump is not None:
+            dump["last_step"] = i == args.steps - 1
         step(True)
     e1.record()
     barrier()
@@ -527,6 +557,13 @@ def run_ours(args):
     kernel_launches_per_step = len(kev) // args.steps
     clocks = sampler.stop() if rank == 0 else None
     flag = flag_of()
+    if dump is not None:
+        if not streamed:
+            dump["values"] = out[tuple(dump["idx"])]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, ("out" if world == 1 else "out_rank%d" % rank) + ".npy"),
+                dump["values"].cpu().numpy())
+        dump = None
 
     t = torch.tensor([ms_total, kernel_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -762,7 +799,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/*.npy (float32, at most 48 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.apply_njobs or args.impl == "reference"):
+        ap.error("--dump-outputs writes the results of --impl ours")
     if args.apply_njobs:
         return run_apply_njobs(args)
     if args.impl == "reference":
