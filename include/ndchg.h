@@ -9,12 +9,30 @@
  * Conradsen et al. (2015) omnibus test on dual-pol covariance time series [C11, Re C12, Im C12, C22].
  * The reference parallelises over rows with OpenMP `prange` (:280); here one GPU thread owns one pixel.
  *
- * `values` is a DEVICE array (rows, cols, k, 4) of float32 or float64 with arbitrary element strides;
- * `result` is a DEVICE uint8 array (rows, cols, k), C-contiguous, written completely (0 / 1).
- * `floating` locals of the reference keep the data type (float32 data -> float32 statistic), its doubles stay
- * double.  The chi-square CDF (GSL's gsl_cdf_chisq_P in the reference) is evaluated in double from the closed
- * forms of the regularised incomplete gamma function for the integer shape 2 (k - 1) the test always has.
- * Asynchronous on `stream`; returns 0 or a negative NDNLM_E* code (message: ndchg_last_error()).
+ * `values` is a DEVICE array (rows, cols, k, bands) of float32 or float64 with arbitrary element strides
+ * (`strides[3]` is the band axis); `result` is a DEVICE uint8 array (rows, cols, k), C-contiguous, written
+ * completely (0 / 1).  Asynchronous on `stream`; every entry returns 0 or a negative NDNLM_E* code (message:
+ * ndchg_last_error()).  Argument checks come before the device-pointer check.
+ *
+ * Dual-pol (ndchg_change_detection, ndchg_omnibus_probability, and NDCHG_POL_DUAL of the _pol entries): bands
+ * [C11, Re C12, Im C12, C22], the reference's arithmetic.  `floating` locals of the reference keep the data type
+ * (float32 data -> float32 statistic), its doubles stay double.  The chi-square CDF (GSL's gsl_cdf_chisq_P in the
+ * reference) is evaluated in double from the closed forms of the regularised incomplete gamma function for the
+ * integer shape 2 (k - 1) the dual-pol test always has.
+ *
+ * Other layouts (the _pol entries), bands on the last axis in this order:
+ *     NDCHG_POL_SINGLE         p = 1   [C11]
+ *     NDCHG_POL_QUAD           p = 3   [C11, Re C12, Im C12, Re C13, Im C13, C22, Re C23, Im C23, C33]
+ *     NDCHG_POL_DUAL_DIAGONAL  p = 2   [C11, C22]            (intensity only)
+ *     NDCHG_POL_QUAD_DIAGONAL  p = 3   [C11, C22, C33]       (intensity only)
+ * The same sequential procedure with lnQ = n (p k ln k + sum_i ln det X_i - k ln det sum_i X_i), z = -2 rho lnQ,
+ * P = P1 + omega2 (P2 - P1), P1 = chi2cdf(z, f), P2 = chi2cdf(z, f + 4).  Full layouts: the reference's
+ * f = (k-1) p^2, rho and omega2 at p.  Diagonal layouts: det = product of the diagonal, f = (k-1) p, rho at p = 1,
+ * omega2 = -f/4 (1 - 1/rho)^2.  Inputs are read in the data type; sums, determinants, logs, rho, omega2, z and the
+ * CDF (regularised incomplete gamma for real shape f/2: series / Legendre continued fraction) are double; only the
+ * returned probability is rounded to the data type.  IEEE rules for degenerate pixels: NaN or all-zero input
+ * gives a NaN statistic, i.e. no change.
+ * Requirements: k >= 2, n >= 1 looks, and n >= 3 for quad-pol (the sample covariance of fewer looks is singular).
  */
 #ifndef NDCHG_H
 #define NDCHG_H
@@ -27,6 +45,12 @@ extern "C" {
 #define NDCHG_F32 0
 #define NDCHG_F64 1
 
+#define NDCHG_POL_DUAL 0
+#define NDCHG_POL_SINGLE 1
+#define NDCHG_POL_QUAD 2
+#define NDCHG_POL_DUAL_DIAGONAL 3
+#define NDCHG_POL_QUAD_DIAGONAL 4
+
 int ndchg_change_detection(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
                            uint8_t* result, double alpha, uint32_t n, void* stream);
 
@@ -34,6 +58,12 @@ int ndchg_change_detection(const void* values, const int64_t shape[3], const int
  * nd/_change.pyx:139-160): `prob` is a DEVICE array (rows, cols) of the data type, C-contiguous. */
 int ndchg_omnibus_probability(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
                               void* prob, uint32_t n, void* stream);
+
+/* The same for the covariance layout `pol` (NDCHG_POL_*); NDCHG_POL_DUAL calls the two entries above. */
+int ndchg_change_detection_pol(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
+                               int pol, uint8_t* result, double alpha, uint32_t n, void* stream);
+int ndchg_omnibus_probability_pol(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
+                                  int pol, void* prob, uint32_t n, void* stream);
 
 const char* ndchg_last_error(void);
 

@@ -32,7 +32,8 @@ SYMBOLS = [
 # every symbol include/ndflt.h declares (sibling filters, SURVEY.md 8(f) row N2)
 FLT_SYMBOLS = ["ndflt_correlate", "ndflt_correlate1d", "ndflt_launch_count", "ndflt_last_error"]
 # every symbol include/ndchg.h declares (omnibus change detection, SURVEY.md 8(f) row N4)
-CHG_SYMBOLS = ["ndchg_change_detection", "ndchg_omnibus_probability", "ndchg_last_error"]
+CHG_SYMBOLS = ["ndchg_change_detection", "ndchg_omnibus_probability", "ndchg_change_detection_pol",
+               "ndchg_omnibus_probability_pol", "ndchg_last_error"]
 
 
 class Info(ctypes.Structure):
@@ -131,6 +132,11 @@ def lib():
     L.ndchg_change_detection.restype = ctypes.c_int
     L.ndchg_omnibus_probability.argtypes = [vp, i64p, i64p, ctypes.c_int, vp, ctypes.c_uint32, vp]
     L.ndchg_omnibus_probability.restype = ctypes.c_int
+    L.ndchg_change_detection_pol.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, vp, ctypes.c_double,
+                                             ctypes.c_uint32, vp]
+    L.ndchg_change_detection_pol.restype = ctypes.c_int
+    L.ndchg_omnibus_probability_pol.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, vp, ctypes.c_uint32, vp]
+    L.ndchg_omnibus_probability_pol.restype = ctypes.c_int
     L.ndchg_last_error.argtypes = []
     L.ndchg_last_error.restype = ctypes.c_char_p
     _lib = L

@@ -6,6 +6,9 @@ Change detection, mirroring reference nd/change.py:13-119 (SURVEY.md 8(f) row N4
 Below `_omnibus_change_detection` the reference calls its Cython / GSL extension `_change.change_detection`
 (nd/_change.pyx:263-287); here that call goes to the CUDA kernel behind include/ndchg.h (one GPU thread per pixel).
 There is no CPU fallback.
+
+Beyond the reference, `pol` selects one of five covariance layouts (`POLS`; include/ndchg.h): dual-pol (the
+reference's path, unchanged), single-pol, quad-pol and the intensity-only dual / quad diagonals.
 """
 import ctypes
 
@@ -19,7 +22,16 @@ from .filters import BoxcarFilter, disassemble_complex
 
 __all__ = ['ChangeDetection', 'OmnibusTest', 'omnibus']
 
-_VARS = ['C11', 'C12__re', 'C12__im', 'C22']
+# covariance layout -> the dataset variables stacked on the last axis, in band order
+POLS = {
+    'dual': ['C11', 'C12__re', 'C12__im', 'C22'],
+    'single': ['C11'],
+    'quad': ['C11', 'C12__re', 'C12__im', 'C13__re', 'C13__im', 'C22', 'C23__re', 'C23__im', 'C33'],
+    'dual_diagonal': ['C11', 'C22'],
+    'quad_diagonal': ['C11', 'C22', 'C33'],
+}
+_POL_CODES = {'dual': 0, 'single': 1, 'quad': 2, 'dual_diagonal': 3, 'quad_diagonal': 4}     # NDCHG_POL_*
+_VARS = POLS['dual']
 
 
 def _check(rc):
@@ -33,10 +45,10 @@ def _check(rc):
     raise RuntimeError('ndchg: ' + msg)
 
 
-def _prepare(values):
+def _prepare(values, bands=4):
     values = np.asarray(values)
-    if values.ndim != 4 or values.shape[3] != 4:
-        raise ValueError('Buffer has wrong number of dimensions (expected (rows, cols, time, 4))')
+    if values.ndim != 4 or values.shape[3] != bands:
+        raise ValueError('Buffer has wrong number of dimensions (expected (rows, cols, time, %d))' % bands)
     if values.dtype not in (np.float32, np.float64):
         raise TypeError('No matching signature found')
     if not torch.cuda.is_available():
@@ -66,6 +78,39 @@ def omnibus_probability(values, n=1):
     return prob.cpu().numpy()
 
 
+def _check_pol(pol, n):
+    if pol not in POLS:
+        raise ValueError('unknown covariance layout pol=%r (one of %s)' % (pol, ', '.join(POLS)))
+    if n < 1 or (pol == 'quad' and n < 3):
+        raise ValueError('pol=%r needs n >= %d looks, got n=%r' % (pol, 3 if pol == 'quad' else 1, n))
+
+
+def change_detection_pol(values, alpha, n=1, pol='dual'):
+    """`change_detection` for the covariance layout `pol` (`POLS`): `values` is (rows, cols, time, bands) with the
+    bands of `POLS[pol]` in that order, multilooked with `n` looks (quad-pol needs n >= 3); returns the uint8 array
+    (rows, cols, time) of detected changes.  `pol='dual'` is `change_detection`."""
+    _check_pol(pol, n)
+    values, t = _prepare(values, len(POLS[pol]))
+    res = torch.empty(values.shape[:3], dtype=torch.uint8, device=t.device)
+    _check(_lib.lib().ndchg_change_detection_pol(ctypes.c_void_p(t.data_ptr()), _lib.i64(values.shape[:3]), _lib.i64(t.stride()),
+                                                 0 if values.dtype == np.float32 else 1, _POL_CODES[pol],
+                                                 ctypes.c_void_p(res.data_ptr()), float(alpha), int(n),
+                                                 ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return res.cpu().numpy()
+
+
+def omnibus_probability_pol(values, n=1, pol='dual'):
+    """`omnibus_probability` for the covariance layout `pol` (see `change_detection_pol`)."""
+    _check_pol(pol, n)
+    values, t = _prepare(values, len(POLS[pol]))
+    prob = torch.empty(values.shape[:2], dtype=t.dtype, device=t.device)
+    _check(_lib.lib().ndchg_omnibus_probability_pol(ctypes.c_void_p(t.data_ptr()), _lib.i64(values.shape[:3]), _lib.i64(t.stride()),
+                                                    0 if values.dtype == np.float32 else 1, _POL_CODES[pol],
+                                                    ctypes.c_void_p(prob.data_ptr()), int(n),
+                                                    ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return prob.cpu().numpy()
+
+
 class ChangeDetection(Algorithm):
     njobs = 1
 
@@ -73,20 +118,31 @@ class ChangeDetection(Algorithm):
         self.njobs = njobs
 
 
-def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1):
-    """Conradsen et al. (2015) omnibus change detection (reference nd/change.py:32-78)."""
+def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None):
+    """Conradsen et al. (2015) omnibus change detection (reference nd/change.py:32-78); `pol` selects the
+    covariance layout (`POLS`, None: the reference's dual-pol path)."""
+    if pol is not None:
+        _check_pol(pol, ml ** 2 if ml is not None else n)
     ds_m = ds.copy(deep=True)
     disassemble_complex(ds_m)
+    if pol is not None:
+        missing = [v for v in POLS[pol] if v not in ds_m.data_vars]
+        if missing:
+            raise ValueError('pol=%r needs the variables %s (complex, or as __re / __im pairs); missing: %s'
+                             % (pol, ', '.join(POLS[pol]), ', '.join(missing)))
     if ml is not None:                                   # multilooking
         ds_m = BoxcarFilter(w=ml).apply(ds_m)
         n = ml ** 2
     dims = ('y', 'x', 'time')
     stack = []
-    for v in _VARS:
+    for v in (_VARS if pol is None else POLS[pol]):
         var = ds_m[v]
         stack.append(np.transpose(var.values, [list(var.dims).index(d) for d in dims]))
     values = np.stack(stack, axis=-1)
-    change = change_detection(values, alpha=alpha, n=n, njobs=njobs)
+    if pol is None:
+        change = change_detection(values, alpha=alpha, n=n, njobs=njobs)
+    else:
+        change = change_detection_pol(values, alpha=alpha, n=n, pol=pol)
     coords = {k: c for k, c in ds.coords.items()}
     return DataArray(np.asarray(change, dtype=bool), dims, coords=coords, attrs=ds.attrs, name='change')
 
@@ -103,16 +159,22 @@ class OmnibusTest(ChangeDetection):
         The number of looks in `ds`; ignored if `ml` is given (default: 1).
     alpha : float (0. ... 1.), optional
         The significance level (default: 0.01).
+    pol : str, optional (keyword only)
+        The covariance layout and the variables it reads: 'dual' (C11, C12, C22), 'single' (C11), 'quad' (C11,
+        C12, C13, C22, C23, C33; needs n >= 3), 'dual_diagonal' (C11, C22) or 'quad_diagonal' (C11, C22, C33).
+        Complex off-diagonals may be given as one complex variable or as `__re` / `__im` pairs.  Default None: the
+        reference's dual-pol path.
     """
 
-    def __init__(self, ml=None, n=1, alpha=0.01, *args, **kwargs):
+    def __init__(self, ml=None, n=1, alpha=0.01, *args, pol=None, **kwargs):
         self.ml = ml
         self.n = n
         self.alpha = alpha
+        self.pol = pol
         super().__init__(*args, **kwargs)
 
     def apply(self, ds):
-        return _omnibus_change_detection(ds, alpha=self.alpha, ml=self.ml, n=self.n, njobs=self.njobs)
+        return _omnibus_change_detection(ds, alpha=self.alpha, ml=self.ml, n=self.n, njobs=self.njobs, pol=self.pol)
 
 
 omnibus = wrap_algorithm(OmnibusTest, 'omnibus')

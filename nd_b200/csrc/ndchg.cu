@@ -2,6 +2,9 @@
 // control flow (nd/_change.pyx:224-260) with the reference's arithmetic types.  The marginal tests of one starting
 // point l grow by one time step at a time, so their sums / determinant product are kept running (the same
 // left-to-right accumulation order as recomputing every subset from scratch, hence identical values).
+// The walk and the probability kernel are templates over the accumulator of one covariance layout: `Acc<T>` is the
+// reference's dual-pol statistic; `AccDiag<T, P>` (single-pol and the diagonal-only layouts) and `AccQuad<T>`
+// (quad-pol) generalise it, reading the data type and computing everything else in double (include/ndchg.h).
 #include "../../include/ndchg.h"
 #include "../../include/ndnlm.h"
 
@@ -81,9 +84,11 @@ __device__ __forceinline__ double omega2_(const double p, const double k, const 
 // running state of `_z` (nd/_change.pyx:45-79) over a growing subset
 template <typename T>
 struct Acc {
+    using value_type = T;
     T c11, c12r, c12i, c22;
     double prod;
     __device__ void reset() { c11 = c12r = c12i = c22 = T(0); prod = 1.0; }
+    __device__ void push(const T* q, const long long s3) { push(q[0], q[s3], q[2 * s3], q[3 * s3]); }
     __device__ void push(const T a, const T br, const T bi, const T d) {
         const T det = sub_(mul_(a, d), add_(mul_(br, br), mul_(bi, bi)));
         prod = __dmul_rn(prod, double(det));
@@ -111,23 +116,134 @@ struct Acc {
     }
 };
 
+// Regularised lower incomplete gamma P(a, y) for REAL a > 0, in double (the layouts other than dual-pol have
+// half-integer shapes): series for y < a + 1, Legendre's continued fraction for Q = 1 - P otherwise (modified Lentz).
+// The algorithm of oracle/gsl_shim/gsl_shim.h; the prefactor exp(-y + a ln y - lgamma(a)) loses ~a ulps, and
+// the probabilities stay within 1e-12 of scipy's up to a = 283.5 (quad-pol, k = 64; tests/test_change_pol.py).
+__device__ double gamma_p(const double a, const double y) {
+    if (isinf(y)) return 1.0;
+    const double lg = lgamma(a);
+    if (y < a + 1.0) {
+        double ap = a, sum = 1.0 / a, del = sum;
+        for (int m = 0; m < 100000; ++m) {
+            ap += 1.0;
+            del *= y / ap;
+            sum += del;
+            if (fabs(del) < fabs(sum) * 1e-17) break;
+        }
+        return sum * exp(-y + a * log(y) - lg);
+    }
+    const double tiny = 1e-300;
+    double b = y + 1.0 - a, c = 1.0 / tiny, d = 1.0 / b, h = d;
+    for (int i = 1; i < 100000; ++i) {
+        const double an = -double(i) * (double(i) - a);
+        b += 2.0;
+        d = an * d + b;
+        if (fabs(d) < tiny) d = tiny;
+        c = b + an / c;
+        if (fabs(c) < tiny) c = tiny;
+        d = 1.0 / d;
+        const double del = d * c;
+        h *= del;
+        if (fabs(del - 1.0) < 1e-16) break;
+    }
+    return 1.0 - exp(-y + a * log(y) - lg) * h;
+}
+
+// chi-square CDF with f = 2 a degrees of freedom; NaN stays NaN, x <= 0 gives 0
+__device__ __forceinline__ double chisq_p_real(const double x, const double a) {
+    if (x != x) return x;
+    if (!(x > 0.0)) return 0.0;
+    return gamma_p(a, 0.5 * x);
+}
+
+// The generalised statistic of the layouts other than dual-pol, in double from the sum of ln det X_i and
+// det sum_i X_i over k steps.  Full covariance (FULL): the reference's f = (k-1) p^2, rho, omega2 at p; diagonal
+// only: f = (k-1) p, rho at p = 1, omega2 = -f/4 (1 - 1/rho)^2 (lnQ is the sum of p single-band lnQs).
+template <int P, bool FULL>
+__device__ __forceinline__ double omnibus_p(const int k, const unsigned n, const double sum_logdet, const double det_of_sum) {
+    const double p = P, kd = double(k), nd = double(n);
+    const double logQ = nd * (p * kd * log(kd) + sum_logdet - kd * log(det_of_sum));
+    const double rho = rho_(FULL ? p : 1.0, kd, nd);
+    const double f = FULL ? (kd - 1.0) * p * p : (kd - 1.0) * p;
+    const double x = 1.0 - 1.0 / rho;
+    const double omega2 = FULL ? omega2_(p, kd, nd, rho) : -f / 4.0 * (x * x);
+    const double z = -2.0 * rho * logQ;
+    const double P1 = chisq_p_real(z, 0.5 * f);
+    const double P2 = chisq_p_real(z, 0.5 * f + 2.0);
+    return P1 + omega2 * (P2 - P1);
+}
+
+// diagonal of a P x P covariance: single-pol (P = 1, where the diagonal and the full statistic coincide) and the
+// intensity-only layouts [C11, C22] / [C11, C22, C33]; det is the product of the diagonal
+template <typename T, int P>
+struct AccDiag {
+    using value_type = T;
+    double c[P];
+    double logdets;
+    __device__ void reset() {
+        for (int b = 0; b < P; ++b) c[b] = 0.0;
+        logdets = 0.0;
+    }
+    __device__ void push(const T* q, const long long s3) {
+        double det = 1.0;
+        for (int b = 0; b < P; ++b) {
+            const double v = double(q[b * s3]);
+            det *= v;
+            c[b] += v;
+        }
+        logdets += log(det);
+    }
+    __device__ T probability(const int k, const unsigned n) const {
+        double det = 1.0;
+        for (int b = 0; b < P; ++b) det *= c[b];
+        return T(omnibus_p<P, P == 1>(k, n, logdets, det));
+    }
+};
+
+// 3 x 3 Hermitian covariance [C11, Re C12, Im C12, Re C13, Im C13, C22, Re C23, Im C23, C33]
 template <typename T>
+struct AccQuad {
+    using value_type = T;
+    double c[9];
+    double logdets;
+    // a, d, g the real diagonal, b = C12, c = C13, e = C23: a d g + 2 Re(b e conj(c)) - a|e|^2 - d|c|^2 - g|b|^2
+    __device__ static double det(const double* m) {
+        const double a = m[0], br = m[1], bi = m[2], cr = m[3], ci = m[4], d = m[5], er = m[6], ei = m[7], g = m[8];
+        const double be_re = br * er - bi * ei, be_im = br * ei + bi * er;
+        return a * d * g + 2.0 * (be_re * cr + be_im * ci) - a * (er * er + ei * ei) - d * (cr * cr + ci * ci) -
+               g * (br * br + bi * bi);
+    }
+    __device__ void reset() {
+        for (int b = 0; b < 9; ++b) c[b] = 0.0;
+        logdets = 0.0;
+    }
+    __device__ void push(const T* q, const long long s3) {
+        double m[9];
+        for (int b = 0; b < 9; ++b) {
+            m[b] = double(q[b * s3]);
+            c[b] += m[b];
+        }
+        logdets += log(det(m));
+    }
+    __device__ T probability(const int k, const unsigned n) const { return T(omnibus_p<3, true>(k, n, logdets, det(c))); }
+};
+
+template <typename A>
 __global__ void __launch_bounds__(128)
-change_detection_kernel(const T* __restrict__ values, const long long rows, const long long cols, const int k,
-                        const long long s0, const long long s1, const long long s2, const long long s3,
+change_detection_kernel(const typename A::value_type* __restrict__ values, const long long rows, const long long cols,
+                        const int k, const long long s0, const long long s1, const long long s2, const long long s3,
                         unsigned char* __restrict__ result, const double alpha, const unsigned n) {
+    using T = typename A::value_type;
     const long long pix = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (pix >= rows * cols) return;
     const long long i = pix / cols, j = pix - i * cols;
     const T* ts = values + i * s0 + j * s1;
     unsigned char* res = result + pix * k;
     for (int t = 0; t < k; ++t) res[t] = 0;
-    auto push = [&](Acc<T>& acc, const int t) {
-        const T* q = ts + (long long)t * s2;
-        acc.push(q[0], q[s3], q[2 * s3], q[3 * s3]);
-    };
+    auto push = [&](A& acc, const int t) { acc.push(ts + (long long)t * s2, s3); };
     int l = 0, r = 0;
-    Acc<T> acc;
+    A acc;
     while (true) {                                                                         // nd/_change.pyx:238-260
         acc.reset();
         for (int t = l; t < k; ++t) push(acc, t);
@@ -147,21 +263,19 @@ change_detection_kernel(const T* __restrict__ values, const long long rows, cons
     }
 }
 
-template <typename T>
+template <typename A>
 __global__ void __launch_bounds__(128)
-omnibus_probability_kernel(const T* __restrict__ values, const long long rows, const long long cols, const int k,
-                           const long long s0, const long long s1, const long long s2, const long long s3,
-                           T* __restrict__ prob, const unsigned n) {
+omnibus_probability_kernel(const typename A::value_type* __restrict__ values, const long long rows, const long long cols,
+                           const int k, const long long s0, const long long s1, const long long s2, const long long s3,
+                           typename A::value_type* __restrict__ prob, const unsigned n) {
+    using T = typename A::value_type;
     const long long pix = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (pix >= rows * cols) return;
     const long long i = pix / cols, j = pix - i * cols;
     const T* ts = values + i * s0 + j * s1;
-    Acc<T> acc;
+    A acc;
     acc.reset();
-    for (int t = 0; t < k; ++t) {
-        const T* q = ts + (long long)t * s2;
-        acc.push(q[0], q[s3], q[2 * s3], q[3 * s3]);
-    }
+    for (int t = 0; t < k; ++t) acc.push(ts + (long long)t * s2, s3);
     prob[pix] = acc.probability(k, n);
 }
 
@@ -195,24 +309,59 @@ static int check_args(const void* values, const int64_t* shape, const int64_t* s
     return NDNLM_OK;
 }
 
+template <typename A>
+static int launch_change(const void* values, const int64_t* shape, const int64_t* strides, uint8_t* result, double alpha,
+                         uint32_t n, void* stream) {
+    const long long pixels = shape[0] * shape[1];
+    const unsigned grid = unsigned((pixels + 127) / 128);
+    ndchg::change_detection_kernel<A><<<grid, 128, 0, (cudaStream_t)stream>>>(
+        (const typename A::value_type*)values, shape[0], shape[1], int(shape[2]), strides[0], strides[1], strides[2],
+        strides[3], result, alpha, n);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+template <typename A>
+static int launch_probability(const void* values, const int64_t* shape, const int64_t* strides, void* prob, uint32_t n,
+                              void* stream) {
+    const long long pixels = shape[0] * shape[1];
+    const unsigned grid = unsigned((pixels + 127) / 128);
+    ndchg::omnibus_probability_kernel<A><<<grid, 128, 0, (cudaStream_t)stream>>>(
+        (const typename A::value_type*)values, shape[0], shape[1], int(shape[2]), strides[0], strides[1], strides[2],
+        strides[3], (typename A::value_type*)prob, n);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+// calls f(A()) with the accumulator of layout `pol` (other than dual-pol, which has its own entry points) for data type T
+template <typename T, typename F>
+static int with_layout(int pol, F&& f) {
+    switch (pol) {
+        case NDCHG_POL_SINGLE: return f(ndchg::AccDiag<T, 1>());
+        case NDCHG_POL_QUAD: return f(ndchg::AccQuad<T>());
+        case NDCHG_POL_DUAL_DIAGONAL: return f(ndchg::AccDiag<T, 2>());
+        case NDCHG_POL_QUAD_DIAGONAL: return f(ndchg::AccDiag<T, 3>());
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+static int check_pol(int pol, uint32_t n) {
+    if (pol < NDCHG_POL_DUAL || pol > NDCHG_POL_QUAD_DIAGONAL) return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    if (pol == NDCHG_POL_QUAD && n < 3)
+        return chg_fail(NDNLM_EINVAL, "quad-pol needs n >= 3 looks (the sample covariance of fewer looks is singular)");
+    return NDNLM_OK;
+}
+
 extern "C" int ndchg_change_detection(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
                                       uint8_t* result, double alpha, uint32_t n, void* stream) {
     int rc = check_args(values, shape, strides, dtype, result, n);
     if (rc) return rc;
     ChgDeviceGuard guard(result);
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "result is not a CUDA device pointer");
-    const long long pixels = shape[0] * shape[1];
-    const unsigned grid = unsigned((pixels + 127) / 128);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == NDCHG_F64)
-        ndchg::change_detection_kernel<double><<<grid, 128, 0, st>>>((const double*)values, shape[0], shape[1], int(shape[2]),
-                                                                    strides[0], strides[1], strides[2], strides[3], result, alpha, n);
-    else
-        ndchg::change_detection_kernel<float><<<grid, 128, 0, st>>>((const float*)values, shape[0], shape[1], int(shape[2]),
-                                                                   strides[0], strides[1], strides[2], strides[3], result, alpha, n);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
-    return NDNLM_OK;
+    if (dtype == NDCHG_F64) return launch_change<ndchg::Acc<double>>(values, shape, strides, result, alpha, n, stream);
+    return launch_change<ndchg::Acc<float>>(values, shape, strides, result, alpha, n, stream);
 }
 
 extern "C" int ndchg_omnibus_probability(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
@@ -221,18 +370,32 @@ extern "C" int ndchg_omnibus_probability(const void* values, const int64_t shape
     if (rc) return rc;
     ChgDeviceGuard guard(prob);
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "prob is not a CUDA device pointer");
-    const long long pixels = shape[0] * shape[1];
-    const unsigned grid = unsigned((pixels + 127) / 128);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == NDCHG_F64)
-        ndchg::omnibus_probability_kernel<double><<<grid, 128, 0, st>>>((const double*)values, shape[0], shape[1], int(shape[2]),
-                                                                       strides[0], strides[1], strides[2], strides[3], (double*)prob, n);
-    else
-        ndchg::omnibus_probability_kernel<float><<<grid, 128, 0, st>>>((const float*)values, shape[0], shape[1], int(shape[2]),
-                                                                      strides[0], strides[1], strides[2], strides[3], (float*)prob, n);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
-    return NDNLM_OK;
+    if (dtype == NDCHG_F64) return launch_probability<ndchg::Acc<double>>(values, shape, strides, prob, n, stream);
+    return launch_probability<ndchg::Acc<float>>(values, shape, strides, prob, n, stream);
+}
+
+extern "C" int ndchg_change_detection_pol(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
+                                          int pol, uint8_t* result, double alpha, uint32_t n, void* stream) {
+    int rc = check_args(values, shape, strides, dtype, result, n);
+    if (!rc) rc = check_pol(pol, n);
+    if (rc) return rc;
+    if (pol == NDCHG_POL_DUAL) return ndchg_change_detection(values, shape, strides, dtype, result, alpha, n, stream);
+    ChgDeviceGuard guard(result);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "result is not a CUDA device pointer");
+    auto go = [&](auto acc) { return launch_change<decltype(acc)>(values, shape, strides, result, alpha, n, stream); };
+    return dtype == NDCHG_F64 ? with_layout<double>(pol, go) : with_layout<float>(pol, go);
+}
+
+extern "C" int ndchg_omnibus_probability_pol(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
+                                             int pol, void* prob, uint32_t n, void* stream) {
+    int rc = check_args(values, shape, strides, dtype, prob, n);
+    if (!rc) rc = check_pol(pol, n);
+    if (rc) return rc;
+    if (pol == NDCHG_POL_DUAL) return ndchg_omnibus_probability(values, shape, strides, dtype, prob, n, stream);
+    ChgDeviceGuard guard(prob);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "prob is not a CUDA device pointer");
+    auto go = [&](auto acc) { return launch_probability<decltype(acc)>(values, shape, strides, prob, n, stream); };
+    return dtype == NDCHG_F64 ? with_layout<double>(pol, go) : with_layout<float>(pol, go);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }

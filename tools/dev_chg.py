@@ -1,36 +1,67 @@
 #!/usr/bin/env python
-"""Development timing (GPU) of the omnibus change-detection kernel: Mpixel/s for a (rows, cols, k, 4) cube."""
-import ctypes, os, sys
+"""Development timing (GPU) of the omnibus change-detection kernels: Mpixel/s for a (rows, cols, k, bands) cube of
+every covariance layout (include/ndchg.h), float32 and float64, with one change per series and without."""
+import ctypes, os, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from nd_b200 import _lib
+from nd_b200 import _lib, change
 
-def run(rows, cols, k, dtype, looks=50, alpha=0.9999, jumps=True):
+P = {'dual': 2, 'single': 1, 'quad': 3, 'dual_diagonal': 2, 'quad_diagonal': 3}
+
+def cube(rows, cols, k, pol, looks, jumps):
+    """n-look sample covariances of independent unit-power channels in the band order of `pol`, generated on the
+    GPU one time step at a time; from k // 2 on the amplitude is x1.5 when `jumps`."""
     g = torch.Generator(device="cuda").manual_seed(0)
-    z = torch.randn((rows, cols, k, looks, 2, 2), device="cuda", generator=g, dtype=torch.float32) / 2 ** 0.5
-    if jumps:
-        z[:, :, k // 2:] *= 1.5
-    zc = torch.complex(z[..., 0], z[..., 1])
-    c11 = (zc[..., 0].abs() ** 2).mean(-1); c22 = (zc[..., 1].abs() ** 2).mean(-1)
-    c12 = (zc[..., 0] * zc[..., 1].conj()).mean(-1)
-    v = torch.stack([c11, c12.real, c12.imag, c22], dim=-1).to(dtype).contiguous()
-    del z, zc
+    out = []
+    for t in range(k):
+        z = torch.randn((rows, cols, looks, P[pol], 2), device="cuda", generator=g) / 2 ** 0.5
+        if jumps and t >= k // 2:
+            z *= 1.5
+        z = torch.complex(z[..., 0], z[..., 1])
+        c = torch.einsum('...li,...lj->...ij', z, z.conj()) / looks
+        if pol == 'dual':
+            b = [c[..., 0, 0].real, c[..., 0, 1].real, c[..., 0, 1].imag, c[..., 1, 1].real]
+        elif pol == 'quad':
+            b = [c[..., 0, 0].real, c[..., 0, 1].real, c[..., 0, 1].imag, c[..., 0, 2].real, c[..., 0, 2].imag,
+                 c[..., 1, 1].real, c[..., 1, 2].real, c[..., 1, 2].imag, c[..., 2, 2].real]
+        else:
+            b = [c[..., i, i].real for i in range(P[pol])]
+        out.append(torch.stack(b, -1))
+    return torch.stack(out, 2)
+
+def run(rows, cols, k, dtype, pol, looks=50, alpha=0.9999, jumps=True):
+    v = cube(rows, cols, k, pol, looks, jumps).to(dtype).contiguous()
     res = torch.empty((rows, cols, k), dtype=torch.uint8, device="cuda")
     L = _lib.lib()
     st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
     def call():
-        rc = L.ndchg_change_detection(ctypes.c_void_p(v.data_ptr()), _lib.i64(v.shape[:3]), _lib.i64(v.stride()),
-                                      0 if dtype == torch.float32 else 1, ctypes.c_void_p(res.data_ptr()), alpha, looks, st)
-        assert rc == 0
+        rc = L.ndchg_change_detection_pol(ctypes.c_void_p(v.data_ptr()), _lib.i64(v.shape[:3]), _lib.i64(v.stride()),
+                                          0 if dtype == torch.float32 else 1, change._POL_CODES[pol],
+                                          ctypes.c_void_p(res.data_ptr()), alpha, looks, st)
+        assert rc == 0, L.ndchg_last_error()
     call(); torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     best = 1e30
     for _ in range(3):
         e0.record(); call(); e1.record(); torch.cuda.synchronize(); best = min(best, e0.elapsed_time(e1))
     nbytes = v.numel() * v.element_size() + res.numel()
-    print("%s %dx%dx%d looks=%d: %.3f ms  %.1f Mpixel/s  %.1f GB/s of algorithmic bytes  changes/pixel=%.3f" % (
-        str(dtype)[6:], rows, cols, k, looks, best, rows * cols / best / 1e3, nbytes / best / 1e6, res.float().sum().item() / (rows * cols)), flush=True)
+    print("%-13s %s %dx%dx%d looks=%d %s: %8.3f ms  %7.1f Mpixel/s  %6.1f GB/s of algorithmic bytes  changes/pixel=%.3f" % (
+        pol, str(dtype)[6:], rows, cols, k, looks, "jumps" if jumps else "flat ", best, rows * cols / best / 1e3,
+        nbytes / best / 1e6, res.float().sum().item() / (rows * cols)), flush=True)
+    del v, res
+    torch.cuda.empty_cache()
 
-run(1024, 1024, 24, torch.float32)
-run(1024, 1024, 24, torch.float64)
-run(1024, 1024, 24, torch.float32, jumps=False)
+def card():
+    try:
+        limit = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
+                                str(torch.cuda.current_device())], capture_output=True, text=True).stdout.strip()
+    except OSError:
+        limit = "unknown"
+    return "%s, power limit %s" % (torch.cuda.get_device_name(), limit or "unknown")
+
+if __name__ == "__main__":
+    print("# %s" % card(), flush=True)
+    for pol in ('dual', 'single', 'quad', 'dual_diagonal', 'quad_diagonal'):
+        for dtype in (torch.float32, torch.float64):
+            for jumps in (True, False):
+                run(1024, 1024, 24, dtype, pol, jumps=jumps)
