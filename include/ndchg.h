@@ -33,6 +33,22 @@
  * returned probability is rounded to the data type.  IEEE rules for degenerate pixels: NaN or all-zero input
  * gives a NaN statistic, i.e. no change.
  * Requirements: k >= 2, n >= 1 looks, and n >= 3 for quad-pol (the sample covariance of fewer looks is singular).
+ *
+ * Direction of each change (ndchg_change_direction): the walk of the layout runs unchanged (NDCHG_POL_DUAL: the
+ * reference's dual-pol walk), then every change is classified by the Loewner order of the covariance after it
+ * against the mean of the segment before it.  With t_1 < t_2 < ... the changes of a pixel and t_0 = 0 (the walk
+ * restarts at each change), for change i: m = t_i - t_{i-1}, S = sum of double(X_s) for s = t_{i-1} .. t_i - 1 per
+ * band, added left to right, M = S / m, D = double(X_t_i) - M, all in double with separate correctly rounded
+ * operations (no FMA).  D is Hermitian, in the band order of the layout:
+ *     single, dual / quad diagonal  increase: every diagonal entry > 0      decrease: every diagonal entry < 0
+ *     dual                          increase: m1 > 0, m2 > 0                decrease: m1 < 0, m2 > 0
+ *     quad                          increase: m1 > 0, m2 > 0, m3 > 0        decrease: m1 < 0, m2 > 0, m3 < 0
+ * with the leading principal minors (Sylvester's criterion) m1 = D11, m2 = D11 D22 - (ReD12 ReD12 + ImD12 ImD12),
+ * m3 = ((a d) g + 2 Re(b e conj(c))) - a |e|^2 - d |c|^2 - g |b|^2 evaluated left to right (a, d, g the diagonal,
+ * b = D12, c = D13, e = D23; Re(b e conj(c)) = (ReB ReE - ImB ImE) ReC + (ReB ImE + ImB ReE) ImC).  Increase means
+ * D is positive definite, decrease negative definite; everything else -- semidefinite, zero, NaN -- is indefinite.
+ * The result holds NDCHG_DIR_NONE where there is no change, so `result != 0` is the change map of
+ * ndchg_change_detection_pol with the same arguments.
  */
 #ifndef NDCHG_H
 #define NDCHG_H
@@ -51,6 +67,11 @@ extern "C" {
 #define NDCHG_POL_DUAL_DIAGONAL 3
 #define NDCHG_POL_QUAD_DIAGONAL 4
 
+#define NDCHG_DIR_NONE 0
+#define NDCHG_DIR_INCREASE 1
+#define NDCHG_DIR_DECREASE 2
+#define NDCHG_DIR_INDEFINITE 3
+
 int ndchg_change_detection(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
                            uint8_t* result, double alpha, uint32_t n, void* stream);
 
@@ -64,6 +85,11 @@ int ndchg_change_detection_pol(const void* values, const int64_t shape[3], const
                                int pol, uint8_t* result, double alpha, uint32_t n, void* stream);
 int ndchg_omnibus_probability_pol(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
                                   int pol, void* prob, uint32_t n, void* stream);
+
+/* ndchg_change_detection_pol followed by the direction of every change: `result` holds NDCHG_DIR_* codes
+ * instead of 0 / 1. */
+int ndchg_change_direction(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                           uint8_t* result, double alpha, uint32_t n, void* stream);
 
 const char* ndchg_last_error(void);
 

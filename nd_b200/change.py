@@ -8,7 +8,8 @@ Below `_omnibus_change_detection` the reference calls its Cython / GSL extension
 There is no CPU fallback.
 
 Beyond the reference, `pol` selects one of five covariance layouts (`POLS`; include/ndchg.h): dual-pol (the
-reference's path, unchanged), single-pol, quad-pol and the intensity-only dual / quad diagonals.
+reference's path, unchanged), single-pol, quad-pol and the intensity-only dual / quad diagonals.  `change_direction`
+and `OmnibusTest(..., direction=True)` also say which way each change went (`DIRECTIONS`).
 """
 import ctypes
 
@@ -32,6 +33,8 @@ POLS = {
 }
 _POL_CODES = {'dual': 0, 'single': 1, 'quad': 2, 'dual_diagonal': 3, 'quad_diagonal': 4}     # NDCHG_POL_*
 _VARS = POLS['dual']
+# codes of `change_direction` (NDCHG_DIR_*): the covariance after a change against the mean of the segment before it
+DIRECTIONS = {'none': 0, 'increase': 1, 'decrease': 2, 'indefinite': 3}
 
 
 def _check(rc):
@@ -111,6 +114,21 @@ def omnibus_probability_pol(values, n=1, pol='dual'):
     return prob.cpu().numpy()
 
 
+def change_direction(values, alpha, n=1, pol='dual'):
+    """`change_detection_pol` that also classifies every change: returns the uint8 array (rows, cols, time) of
+    `DIRECTIONS` codes -- 0 no change, 1 increase (the covariance minus the mean of the segment since the previous
+    change is positive definite), 2 decrease (negative definite), 3 indefinite (a mixed change, include/ndchg.h).
+    `result != 0` is the change map of `change_detection_pol`; `pol='dual'` walks the reference's dual-pol path."""
+    _check_pol(pol, n)
+    values, t = _prepare(values, len(POLS[pol]))
+    res = torch.empty(values.shape[:3], dtype=torch.uint8, device=t.device)
+    _check(_lib.lib().ndchg_change_direction(ctypes.c_void_p(t.data_ptr()), _lib.i64(values.shape[:3]), _lib.i64(t.stride()),
+                                             0 if values.dtype == np.float32 else 1, _POL_CODES[pol],
+                                             ctypes.c_void_p(res.data_ptr()), float(alpha), int(n),
+                                             ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return res.cpu().numpy()
+
+
 class ChangeDetection(Algorithm):
     njobs = 1
 
@@ -118,9 +136,9 @@ class ChangeDetection(Algorithm):
         self.njobs = njobs
 
 
-def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None):
+def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None, direction=False):
     """Conradsen et al. (2015) omnibus change detection (reference nd/change.py:32-78); `pol` selects the
-    covariance layout (`POLS`, None: the reference's dual-pol path)."""
+    covariance layout (`POLS`, None: the reference's dual-pol path); `direction` returns `DIRECTIONS` codes."""
     if pol is not None:
         _check_pol(pol, ml ** 2 if ml is not None else n)
     ds_m = ds.copy(deep=True)
@@ -139,11 +157,14 @@ def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None):
         var = ds_m[v]
         stack.append(np.transpose(var.values, [list(var.dims).index(d) for d in dims]))
     values = np.stack(stack, axis=-1)
+    coords = {k: c for k, c in ds.coords.items()}
+    if direction:                                        # pol=None: the reference's walk, through the 'dual' entry
+        codes = change_direction(values, alpha=alpha, n=n, pol='dual' if pol is None else pol)
+        return DataArray(codes, dims, coords=coords, attrs=ds.attrs, name='change_direction')
     if pol is None:
         change = change_detection(values, alpha=alpha, n=n, njobs=njobs)
     else:
         change = change_detection_pol(values, alpha=alpha, n=n, pol=pol)
-    coords = {k: c for k, c in ds.coords.items()}
     return DataArray(np.asarray(change, dtype=bool), dims, coords=coords, attrs=ds.attrs, name='change')
 
 
@@ -164,17 +185,23 @@ class OmnibusTest(ChangeDetection):
         C12, C13, C22, C23, C33; needs n >= 3), 'dual_diagonal' (C11, C22) or 'quad_diagonal' (C11, C22, C33).
         Complex off-diagonals may be given as one complex variable or as `__re` / `__im` pairs.  Default None: the
         reference's dual-pol path.
+    direction : bool, optional (keyword only)
+        If True, `apply` returns uint8 codes named 'change_direction' instead of the boolean 'change': 0 no
+        change, 1 increase, 2 decrease, 3 indefinite (`DIRECTIONS`; computed on the multilooked values when `ml`
+        is given).  Default False.
     """
 
-    def __init__(self, ml=None, n=1, alpha=0.01, *args, pol=None, **kwargs):
+    def __init__(self, ml=None, n=1, alpha=0.01, *args, pol=None, direction=False, **kwargs):
         self.ml = ml
         self.n = n
         self.alpha = alpha
         self.pol = pol
+        self.direction = direction
         super().__init__(*args, **kwargs)
 
     def apply(self, ds):
-        return _omnibus_change_detection(ds, alpha=self.alpha, ml=self.ml, n=self.n, njobs=self.njobs, pol=self.pol)
+        return _omnibus_change_detection(ds, alpha=self.alpha, ml=self.ml, n=self.n, njobs=self.njobs, pol=self.pol,
+                                         direction=self.direction)
 
 
 omnibus = wrap_algorithm(OmnibusTest, 'omnibus')

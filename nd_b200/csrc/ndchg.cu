@@ -5,6 +5,8 @@
 // The walk and the probability kernel are templates over the accumulator of one covariance layout: `Acc<T>` is the
 // reference's dual-pol statistic; `AccDiag<T, P>` (single-pol and the diagonal-only layouts) and `AccQuad<T>`
 // (quad-pol) generalise it, reading the data type and computing everything else in double (include/ndchg.h).
+// `change_direction_kernel` is a post-pass over the walk's change map that classifies each change as an increase,
+// a decrease or indefinite; the walk kernels do not know about it.
 #include "../../include/ndchg.h"
 #include "../../include/ndnlm.h"
 
@@ -279,6 +281,85 @@ omnibus_probability_kernel(const typename A::value_type* __restrict__ values, co
     prob[pix] = acc.probability(k, n);
 }
 
+// Loewner order of D = X_t - mean of the segment before it (include/ndchg.h).  Every operation is a separate,
+// correctly rounded double operation in the order of oracle/omnibus_direction_oracle.py::classify, so the codes match the
+// oracle exactly; AccQuad::det is deliberately not reused (written without intrinsics, nvcc contracts it into FMAs).
+__host__ __device__ constexpr int pol_bands(const int pol) {
+    return pol == NDCHG_POL_DUAL ? 4 : pol == NDCHG_POL_SINGLE ? 1 : pol == NDCHG_POL_QUAD ? 9 : pol == NDCHG_POL_DUAL_DIAGONAL ? 2 : 3;
+}
+
+template <int POL>
+__device__ __forceinline__ unsigned char classify(const double* D) {
+    if constexpr (POL == NDCHG_POL_DUAL || POL == NDCHG_POL_QUAD) {
+        // Sylvester's criterion on the leading principal minors; C22 is band 3 (dual) or 5 (quad)
+        constexpr int i22 = POL == NDCHG_POL_DUAL ? 3 : 5;
+        const double m1 = D[0];
+        const double m2 = __dsub_rn(__dmul_rn(D[0], D[i22]), __dadd_rn(__dmul_rn(D[1], D[1]), __dmul_rn(D[2], D[2])));
+        if constexpr (POL == NDCHG_POL_DUAL) {
+            if (m1 > 0.0 && m2 > 0.0) return NDCHG_DIR_INCREASE;
+            if (m1 < 0.0 && m2 > 0.0) return NDCHG_DIR_DECREASE;
+        } else {
+            const double a = D[0], br = D[1], bi = D[2], cr = D[3], ci = D[4], d = D[5], er = D[6], ei = D[7], g = D[8];
+            // ((a*d)*g + 2*re_bec) - a*(|e|^2) - d*(|c|^2) - g*(|b|^2), re_bec = Re(b e conj(c))
+            const double re_bec = __dadd_rn(__dmul_rn(__dsub_rn(__dmul_rn(br, er), __dmul_rn(bi, ei)), cr),
+                                            __dmul_rn(__dadd_rn(__dmul_rn(br, ei), __dmul_rn(bi, er)), ci));
+            double m3 = __dadd_rn(__dmul_rn(__dmul_rn(a, d), g), __dmul_rn(2.0, re_bec));
+            m3 = __dsub_rn(m3, __dmul_rn(a, __dadd_rn(__dmul_rn(er, er), __dmul_rn(ei, ei))));
+            m3 = __dsub_rn(m3, __dmul_rn(d, __dadd_rn(__dmul_rn(cr, cr), __dmul_rn(ci, ci))));
+            m3 = __dsub_rn(m3, __dmul_rn(g, __dadd_rn(__dmul_rn(br, br), __dmul_rn(bi, bi))));
+            if (m1 > 0.0 && m2 > 0.0 && m3 > 0.0) return NDCHG_DIR_INCREASE;
+            if (m1 < 0.0 && m2 > 0.0 && m3 < 0.0) return NDCHG_DIR_DECREASE;
+        }
+        return NDCHG_DIR_INDEFINITE;
+    } else {
+        // single and the intensity-only diagonals: signs of the diagonal, no products (nothing can underflow)
+        bool up = true, down = true;
+        for (int b = 0; b < pol_bands(POL); ++b) {
+            up = up && D[b] > 0.0;
+            down = down && D[b] < 0.0;
+        }
+        return up ? NDCHG_DIR_INCREASE : down ? NDCHG_DIR_DECREASE : NDCHG_DIR_INDEFINITE;
+    }
+}
+
+// Post-pass after change_detection_kernel on the same stream: rewrites each pixel's 0 / 1 change vector in place
+// with the direction codes.  A pixel without a change returns before reading `values`; otherwise its series is read
+// once, up to its last change.  The segment before a change starts at the previous change (the walk restarts there).
+template <typename T, int POL>
+__global__ void __launch_bounds__(128)
+change_direction_kernel(const T* __restrict__ values, const long long rows, const long long cols, const int k,
+                        const long long s0, const long long s1, const long long s2, const long long s3,
+                        unsigned char* __restrict__ result) {
+    constexpr int B = pol_bands(POL);
+    const long long pix = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= rows * cols) return;
+    unsigned char* res = result + pix * k;
+    int last = -1;
+    for (int t = 0; t < k; ++t)
+        if (res[t]) last = t;
+    if (last < 0) return;
+    const long long i = pix / cols, j = pix - i * cols;
+    const T* ts = values + i * s0 + j * s1;
+    double S[B];
+    for (int b = 0; b < B; ++b) S[b] = 0.0;
+    int m = 0;
+    for (int t = 0; t <= last; ++t) {
+        const T* q = ts + (long long)t * s2;
+        if (res[t]) {                                        // the walk never marks t = 0, so m >= 1 here
+            double D[B];
+            const double md = double(m);
+            for (int b = 0; b < B; ++b) {
+                D[b] = __dsub_rn(double(q[b * s3]), __ddiv_rn(S[b], md));
+                S[b] = 0.0;
+            }
+            res[t] = classify<POL>(D);
+            m = 0;
+        }
+        for (int b = 0; b < B; ++b) S[b] = __dadd_rn(S[b], double(q[b * s3]));
+        ++m;
+    }
+}
+
 }  // namespace ndchg
 
 struct ChgDeviceGuard {
@@ -396,6 +477,43 @@ extern "C" int ndchg_omnibus_probability_pol(const void* values, const int64_t s
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "prob is not a CUDA device pointer");
     auto go = [&](auto acc) { return launch_probability<decltype(acc)>(values, shape, strides, prob, n, stream); };
     return dtype == NDCHG_F64 ? with_layout<double>(pol, go) : with_layout<float>(pol, go);
+}
+
+template <typename T, int POL>
+static int launch_direction(const void* values, const int64_t* shape, const int64_t* strides, uint8_t* result, void* stream) {
+    const long long pixels = shape[0] * shape[1];
+    const unsigned grid = unsigned((pixels + 127) / 128);
+    ndchg::change_direction_kernel<T, POL><<<grid, 128, 0, (cudaStream_t)stream>>>(
+        (const T*)values, shape[0], shape[1], int(shape[2]), strides[0], strides[1], strides[2], strides[3], result);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+template <typename T>
+static int launch_direction(int pol, const void* values, const int64_t* shape, const int64_t* strides, uint8_t* result,
+                            void* stream) {
+    switch (pol) {
+        case NDCHG_POL_DUAL: return launch_direction<T, NDCHG_POL_DUAL>(values, shape, strides, result, stream);
+        case NDCHG_POL_SINGLE: return launch_direction<T, NDCHG_POL_SINGLE>(values, shape, strides, result, stream);
+        case NDCHG_POL_QUAD: return launch_direction<T, NDCHG_POL_QUAD>(values, shape, strides, result, stream);
+        case NDCHG_POL_DUAL_DIAGONAL: return launch_direction<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, result, stream);
+        case NDCHG_POL_QUAD_DIAGONAL: return launch_direction<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, result, stream);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+extern "C" int ndchg_change_direction(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype,
+                                      int pol, uint8_t* result, double alpha, uint32_t n, void* stream) {
+    int rc = check_args(values, shape, strides, dtype, result, n);
+    if (!rc) rc = check_pol(pol, n);
+    if (rc) return rc;
+    ChgDeviceGuard guard(result);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "result is not a CUDA device pointer");
+    rc = ndchg_change_detection_pol(values, shape, strides, dtype, pol, result, alpha, n, stream);
+    if (rc) return rc;
+    return dtype == NDCHG_F64 ? launch_direction<double>(pol, values, shape, strides, result, stream)
+                              : launch_direction<float>(pol, values, shape, strides, result, stream);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }
