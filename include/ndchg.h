@@ -91,6 +91,29 @@ int ndchg_omnibus_probability_pol(const void* values, const int64_t shape[3], co
 int ndchg_change_direction(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
                            uint8_t* result, double alpha, uint32_t n, void* stream);
 
+/* Equivalent number of looks of every sample, estimated over a square window of odd side `window` (3 <= window <=
+ * min(rows, cols)) in (rows, cols); each time step on its own.  `values` as above, in the band order of `pol`; `enl`
+ * is a DEVICE array (rows, cols, k) of the data type, C-contiguous, written completely.  Requires k >= 1.
+ *
+ * With N = window^2 and l = ln det X of every sample (det of the layout: the 2 x 2 / 3 x 3 Hermitian determinant,
+ * the product of the diagonal for the diagonal layouts), for a pixel whose window lies inside the image:
+ *     M = the band-wise mean over the window,   delta = ln det M - (mean of l over the window),
+ * and the ENL is the root L of h(L) = G(L) - G(N L) = delta, where
+ *     full layouts (single, dual, quad; d = p):  G(L) = d ln L - sum_{i=0}^{d-1} psi(L - i)   on L > d - 1,
+ *     diagonal layouts (independent Gamma channels with a common L):  G(L) = p (ln L - psi(L))   on L > 0.
+ * For an L-look complex Wishart sample E[ln det X] = ln det Sigma + sum_i psi(L - i) - d ln L, and the window mean of
+ * N independent samples has N L looks, so E[delta] = G(L) - G(N L) exactly (no small-window bias; N -> infinity is
+ * the maximum-likelihood estimator of Anfinsen et al., IEEE TGRS 2009).  h falls strictly from +inf to 0, so the
+ * root is unique.  Textured (non-homogeneous) windows bias L low; spatially correlated samples (box means, filtered
+ * data) bias it high, since the estimator takes the N samples of a window as independent.
+ * Edge rules: pixels within window / 2 of the image border are NaN; a window containing a sample with a non-finite
+ * band or det <= 0 is NaN (as is a window whose mean has det <= 0); delta <= 0 (no speckle) gives +inf.
+ * Arithmetic: inputs are read in the data type, everything else is double (psi and psi' by recurrence and the
+ * asymptotic series); window sums are direct sums of window^2 terms; the root is found by Newton's method inside a
+ * bracket to a relative 1e-13 and rounded once to the data type. */
+int ndchg_enl(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol, uint32_t window,
+              void* enl, void* stream);
+
 const char* ndchg_last_error(void);
 
 #ifdef __cplusplus

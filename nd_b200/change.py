@@ -9,7 +9,9 @@ There is no CPU fallback.
 
 Beyond the reference, `pol` selects one of five covariance layouts (`POLS`; include/ndchg.h): dual-pol (the
 reference's path, unchanged), single-pol, quad-pol and the intensity-only dual / quad diagonals.  `change_direction`
-and `OmnibusTest(..., direction=True)` also say which way each change went (`DIRECTIONS`).
+and `OmnibusTest(..., direction=True)` also say which way each change went (`DIRECTIONS`).  `enl_map`,
+`EquivalentLooks` / `equivalent_looks` estimate the equivalent number of looks from the data, and
+`OmnibusTest(n='auto')` uses that estimate as the test's number of looks.
 """
 import ctypes
 
@@ -21,7 +23,7 @@ from .algorithm import Algorithm, wrap_algorithm
 from .dataset import DataArray
 from .filters import BoxcarFilter, disassemble_complex
 
-__all__ = ['ChangeDetection', 'OmnibusTest', 'omnibus']
+__all__ = ['ChangeDetection', 'OmnibusTest', 'omnibus', 'EquivalentLooks', 'equivalent_looks', 'enl_map']
 
 # covariance layout -> the dataset variables stacked on the last axis, in band order
 POLS = {
@@ -81,9 +83,13 @@ def omnibus_probability(values, n=1):
     return prob.cpu().numpy()
 
 
-def _check_pol(pol, n):
+def _check_layout(pol):
     if pol not in POLS:
         raise ValueError('unknown covariance layout pol=%r (one of %s)' % (pol, ', '.join(POLS)))
+
+
+def _check_pol(pol, n):
+    _check_layout(pol)
     if n < 1 or (pol == 'quad' and n < 3):
         raise ValueError('pol=%r needs n >= %d looks, got n=%r' % (pol, 3 if pol == 'quad' else 1, n))
 
@@ -129,18 +135,29 @@ def change_direction(values, alpha, n=1, pol='dual'):
     return res.cpu().numpy()
 
 
-class ChangeDetection(Algorithm):
-    njobs = 1
+def enl_map(values, window=7, pol='dual'):
+    """Equivalent number of looks of every sample (include/ndchg.h, `ndchg_enl`): `values` is (rows, cols, time,
+    bands) with the bands of `POLS[pol]`; each time step is estimated over a `window` x `window` neighbourhood (odd,
+    3 <= window <= min(rows, cols)).  Returns (rows, cols, time) in the data type: NaN within window // 2 of the
+    border and where a window holds a non-finite or non-positive-definite sample, +inf where a window has no
+    speckle.  Textured windows bias the estimate low; for a scene ENL take the median over a homogeneous area."""
+    _check_layout(pol)
+    values = np.asarray(values)
+    if isinstance(window, bool) or int(window) != window or window < 3 or window % 2 == 0:
+        raise ValueError('the window must be an odd integer >= 3, got %r' % (window,))
+    if values.ndim == 4 and window > min(values.shape[:2]):
+        raise ValueError('the window (%d) must not exceed the image (%d x %d)' % (window, values.shape[0], values.shape[1]))
+    values, t = _prepare(values, len(POLS[pol]))
+    enl = torch.empty(values.shape[:3], dtype=t.dtype, device=t.device)
+    _check(_lib.lib().ndchg_enl(ctypes.c_void_p(t.data_ptr()), _lib.i64(values.shape[:3]), _lib.i64(t.stride()),
+                                0 if values.dtype == np.float32 else 1, _POL_CODES[pol], int(window),
+                                ctypes.c_void_p(enl.data_ptr()), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return enl.cpu().numpy()
 
-    def __init__(self, njobs=1):
-        self.njobs = njobs
 
-
-def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None, direction=False):
-    """Conradsen et al. (2015) omnibus change detection (reference nd/change.py:32-78); `pol` selects the
-    covariance layout (`POLS`, None: the reference's dual-pol path); `direction` returns `DIRECTIONS` codes."""
-    if pol is not None:
-        _check_pol(pol, ml ** 2 if ml is not None else n)
+def _stack(ds, pol, ml=None):
+    """The variables of layout `pol` (None: the reference's dual-pol variables) as (y, x, time, bands), multilooked
+    with an `ml` x `ml` boxcar when `ml` is given."""
     ds_m = ds.copy(deep=True)
     disassemble_complex(ds_m)
     if pol is not None:
@@ -150,22 +167,99 @@ def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None, d
                              % (pol, ', '.join(POLS[pol]), ', '.join(missing)))
     if ml is not None:                                   # multilooking
         ds_m = BoxcarFilter(w=ml).apply(ds_m)
-        n = ml ** 2
-    dims = ('y', 'x', 'time')
     stack = []
     for v in (_VARS if pol is None else POLS[pol]):
         var = ds_m[v]
-        stack.append(np.transpose(var.values, [list(var.dims).index(d) for d in dims]))
-    values = np.stack(stack, axis=-1)
+        stack.append(np.transpose(var.values, [list(var.dims).index(d) for d in _DIMS]))
+    return np.stack(stack, axis=-1)
+
+
+_DIMS = ('y', 'x', 'time')
+_AUTO_WINDOW = 7                                         # window of the ENL estimate behind n='auto'
+
+
+def _auto_looks(values, pol, ml=None):
+    """n='auto': E = the median ENL of `values` over all pixels and steps, times ml**2 when `values` are the data
+    before an ml x ml boxcar, and the looks max(floor(E), 1) (3 for quad-pol); the walk takes integer looks.
+    With `ml` the estimate is not taken on the multilooked values: neighbouring boxcar outputs share their input
+    samples, so a window of them is not N independent samples and the estimator would overstate the looks."""
+    enl = enl_map(values, _AUTO_WINDOW, 'dual' if pol is None else pol)
+    E = float('nan') if np.isnan(enl).all() else float(np.nanmedian(enl))
+    if not np.isfinite(E):
+        hint = ("; with ml, single-look data of a full covariance layout have singular samples: leave n out to use "
+                "n = ml**2" if ml is not None else "; pass n explicitly")
+        raise ValueError("n='auto': the equivalent number of looks could not be estimated from the data (median %r)%s"
+                         % (E, hint))
+    if ml is not None:
+        E *= ml ** 2
+    return E, max(int(np.floor(E)), 3 if pol == 'quad' else 1)
+
+
+class EquivalentLooks(Algorithm):
+    """
+    Equivalent number of looks of every pixel and time step of a covariance time series (`enl_map`).
+
+    Parameters
+    ----------
+    window : int, optional
+        Side of the square (y, x) window of each estimate, odd and >= 3 (default: 7).
+    pol : str, optional (keyword only)
+        The covariance layout and the variables it reads, as for `OmnibusTest` (default None: dual-pol C11, C12, C22).
+
+    `apply(ds)` returns a DataArray 'enl' over ('y', 'x', 'time') with the dataset's coords and attrs.  Textured
+    areas bias the estimate low: apply it to a homogeneous subset and take the median for a scene ENL.
+    """
+
+    def __init__(self, window=7, *, pol=None):
+        self.window = window
+        self.pol = pol
+
+    def apply(self, ds):
+        if self.pol is not None:
+            _check_layout(self.pol)
+        enl = enl_map(_stack(ds, self.pol), self.window, 'dual' if self.pol is None else self.pol)
+        return DataArray(enl, _DIMS, coords={k: c for k, c in ds.coords.items()}, attrs=ds.attrs, name='enl')
+
+
+equivalent_looks = wrap_algorithm(EquivalentLooks, 'equivalent_looks')
+
+
+class ChangeDetection(Algorithm):
+    njobs = 1
+
+    def __init__(self, njobs=1):
+        self.njobs = njobs
+
+
+def _omnibus_change_detection(ds, alpha=0.01, ml=None, n=1, njobs=1, pol=None, direction=False):
+    """Conradsen et al. (2015) omnibus change detection (reference nd/change.py:32-78); `pol` selects the
+    covariance layout (`POLS`, None: the reference's dual-pol path); `direction` returns `DIRECTIONS` codes;
+    n='auto' estimates the looks of the values the walk reads and records them in the result's attrs."""
+    auto = isinstance(n, str)
+    if auto and n != 'auto':
+        raise ValueError("n must be a number of looks or 'auto', got %r" % (n,))
+    if pol is not None:
+        if auto:
+            _check_layout(pol)
+        else:
+            _check_pol(pol, ml ** 2 if ml is not None else n)
+    values = _stack(ds, pol, ml)
+    attrs = ds.attrs
+    if auto:
+        E, n = _auto_looks(values if ml is None else _stack(ds, pol), pol, ml)
+        attrs = dict(ds.attrs, enl=E, looks=n)
+    elif ml is not None:
+        n = ml ** 2
+    dims = _DIMS
     coords = {k: c for k, c in ds.coords.items()}
     if direction:                                        # pol=None: the reference's walk, through the 'dual' entry
         codes = change_direction(values, alpha=alpha, n=n, pol='dual' if pol is None else pol)
-        return DataArray(codes, dims, coords=coords, attrs=ds.attrs, name='change_direction')
+        return DataArray(codes, dims, coords=coords, attrs=attrs, name='change_direction')
     if pol is None:
         change = change_detection(values, alpha=alpha, n=n, njobs=njobs)
     else:
         change = change_detection_pol(values, alpha=alpha, n=n, pol=pol)
-    return DataArray(np.asarray(change, dtype=bool), dims, coords=coords, attrs=ds.attrs, name='change')
+    return DataArray(np.asarray(change, dtype=bool), dims, coords=coords, attrs=attrs, name='change')
 
 
 class OmnibusTest(ChangeDetection):
@@ -176,8 +270,13 @@ class OmnibusTest(ChangeDetection):
     ----------
     ml : int, optional
         Multilooking window size (default: the dataset is already multilooked).
-    n : int, optional
-        The number of looks in `ds`; ignored if `ml` is given (default: 1).
+    n : int or 'auto', optional
+        The number of looks in `ds`; an integer is ignored if `ml` is given, which uses ml**2 (default: 1).
+        'auto' estimates it: E = the median of `enl_map` with a 7 x 7 window over all pixels and steps of `ds`,
+        times ml**2 when `ml` is given (the estimate is taken before the boxcar, whose outputs are correlated), then
+        n = max(floor(E), 1) (3 for quad-pol); the result's attrs gain 'enl' = E and 'looks' = n.  The estimate
+        assumes mostly homogeneous scenes and spatially uncorrelated input pixels: texture biases it low (a
+        conservative test); spatially correlated input, e.g. data that were already filtered, biases it high.
     alpha : float (0. ... 1.), optional
         The significance level (default: 0.01).
     pol : str, optional (keyword only)

@@ -14,6 +14,7 @@
 #include <cstdio>
 
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 static thread_local char g_chg_err[512] = "";
 static int chg_fail(int code, const char* fmt, ...) {
@@ -360,6 +361,189 @@ change_direction_kernel(const T* __restrict__ values, const long long rows, cons
     }
 }
 
+// ---- equivalent number of looks (ndchg_enl, include/ndchg.h) -----------------------------------------------------
+// g(L, s) = ln L - psi(L - s) and dg = d/dL g = 1/L - psi'(L - s), for L - s > 0: psi and psi' by the recurrence
+// psi(x) = psi(x + m) - sum_{j<m} 1/(x + j) up to y = x + m >= 10, then the asymptotic series of ln y - psi(y) and
+// psi'(y) (Bernoulli numbers up to B14; the first omitted term is < 5e-17 at y = 10).  ln L - ln y is formed as
+// -log1p((m - s) / L), so g keeps its relative accuracy at large L, where it is ~ (s + 1/2) / L and the plain
+// difference ln L - psi(L - s) would cancel.
+__device__ __forceinline__ void ln_minus_digamma(const double L, const int s, double& g, double& dg) {
+    const double x = L - double(s);
+    double r = 0.0, r2 = 0.0;
+    int m = 0;
+    while (x + double(m) < 10.0) {
+        const double inv = 1.0 / (x + double(m));
+        r += inv;
+        r2 += inv * inv;
+        ++m;
+    }
+    const double iy = 1.0 / (x + double(m)), iy2 = iy * iy;
+    // ln y - psi(y) = 1/(2y) + 1/(12y^2) - 1/(120y^4) + 1/(252y^6) - 1/(240y^8) + 1/(132y^10) - 691/(32760y^12) + 1/(12y^14)
+    const double lnpsi = 0.5 * iy + iy2 * (1.0 / 12 + iy2 * (-1.0 / 120 + iy2 * (1.0 / 252 + iy2 * (-1.0 / 240 +
+                         iy2 * (1.0 / 132 + iy2 * (-691.0 / 32760 + iy2 * (1.0 / 12)))))));
+    // psi'(y) = 1/y + 1/(2y^2) + 1/(6y^3) - 1/(30y^5) + 1/(42y^7) - 1/(30y^9) + 5/(66y^11) - 691/(2730y^13) + 7/(6y^15)
+    const double trigamma = iy + iy2 * (0.5 + iy * (1.0 / 6 + iy2 * (-1.0 / 30 + iy2 * (1.0 / 42 + iy2 * (-1.0 / 30 +
+                            iy2 * (5.0 / 66 + iy2 * (-691.0 / 2730 + iy2 * (7.0 / 6))))))));
+    g = -log1p(double(m - s) / L) + r + lnpsi;
+    dg = 1.0 / L - (trigamma + r2);
+}
+
+// G(L) and G'(L): full layouts (p x p complex Wishart) G = sum_{i<P} (ln L - psi(L - i)) on L > P - 1; diagonal
+// layouts (P independent Gamma channels) G = P (ln L - psi(L)) on L > 0.
+template <int P, bool FULL>
+__device__ __forceinline__ void enl_G(const double L, double& G, double& dG) {
+    if constexpr (FULL) {
+        G = dG = 0.0;
+        for (int i = 0; i < P; ++i) {
+            double g, dg;
+            ln_minus_digamma(L, i, g, dg);
+            G += g;
+            dG += dg;
+        }
+    } else {
+        ln_minus_digamma(L, 0, G, dG);
+        G *= P;
+        dG *= P;
+    }
+}
+
+// The root of h(L) = G(L) - G(N L) = delta (h falls strictly from +inf to 0 on the domain), to a relative 1e-13:
+// Newton from the large-L approximation h ~ c (1 - 1/N) / L (c = P^2 / 2 full, P / 2 diagonal), kept inside the
+// bracket [lo, hi] of the iterates seen so far (bisection, or doubling while no upper bound is known).
+template <int P, bool FULL>
+__device__ double enl_solve(const double delta, const double N) {
+    double lo = FULL ? double(P - 1) : 0.0, hi = CUDART_INF;
+    const double c = FULL ? 0.5 * P * P : 0.5 * P;
+    double L = lo + c * (1.0 - 1.0 / N) / delta;
+    for (int it = 0; it < 200; ++it) {
+        double G1, dG1, GN, dGN;
+        enl_G<P, FULL>(L, G1, dG1);
+        enl_G<P, FULL>(N * L, GN, dGN);
+        const double f = (G1 - GN) - delta, df = dG1 - N * dGN;
+        if (f == 0.0) return L;
+        if (f > 0.0) lo = L;
+        else hi = L;
+        double next = L - f / df;
+        if (!(next > lo && next < hi)) next = isinf(hi) ? 2.0 * L : 0.5 * (lo + hi);
+        if (fabs(next - L) <= 1e-13 * next || hi - lo <= 1e-15 * lo) return next;
+        L = next;
+    }
+    return L;
+}
+
+// One CTA: an output tile of ENL_TR x ENL_TC pixels x KT time steps.  The input rows of the tile plus the w - 1
+// halo rows are read one at a time, in segments of ENL_SEG pixels; a thread per sample reads its bands (contiguous
+// for C-contiguous input, as are the KT samples of a pixel), forms ln det and stores the B + 1 doubles in shared
+// memory.  The horizontal window sums of the row (w terms each, added left to right) go to H and are added to the
+// vertical sums V of every output row whose window contains the input row, in row order: each window sum is a
+// direct sum of w x w terms, never a running add / subtract.  Then every thread solves its outputs.
+constexpr int ENL_TR = 16, ENL_TC = 32, ENL_SEG = 64, ENL_THREADS = 256;
+
+template <typename T, int POL>
+struct EnlTile {
+    static constexpr int B = pol_bands(POL);
+    static constexpr int E = B + 1;                                      // bands, then ln det
+    static constexpr int KT = (32 / int(sizeof(T)) + B - 1) / B;         // >= 32 bytes of each pixel per row read
+    static constexpr size_t smem = sizeof(double) * E * KT * (size_t(ENL_TR) * ENL_TC + ENL_TC + ENL_SEG);
+};
+
+template <int POL>
+__device__ __forceinline__ double sample_det(const double* x) {
+    if constexpr (POL == NDCHG_POL_DUAL) {
+        return x[0] * x[3] - (x[1] * x[1] + x[2] * x[2]);
+    } else if constexpr (POL == NDCHG_POL_QUAD) {
+        return AccQuad<double>::det(x);
+    } else {
+        double d = 1.0;
+        for (int b = 0; b < pol_bands(POL); ++b) d *= x[b];
+        return d;
+    }
+}
+
+template <typename T, int POL>
+__global__ void __launch_bounds__(ENL_THREADS)
+enl_kernel(const T* __restrict__ values, const long long rows, const long long cols, const int k, const long long s0,
+           const long long s1, const long long s2, const long long s3, const int w, T* __restrict__ enl) {
+    using Tile = EnlTile<T, POL>;
+    constexpr int B = Tile::B, E = Tile::E, KT = Tile::KT;
+    extern __shared__ double smem[];
+    double* V = smem;                                                    // [ENL_TR][ENL_TC][KT][E]
+    double* H = V + ENL_TR * ENL_TC * KT * E;                            // [ENL_TC][KT][E]
+    double* S = H + ENL_TC * KT * E;                                     // [ENL_SEG][KT][E]
+    const int tid = threadIdx.x, hw = w / 2;
+    const int t0 = blockIdx.x * KT;
+    const long long j0 = (long long)blockIdx.y * ENL_TC, i0 = (long long)blockIdx.z * ENL_TR;
+    for (int e = tid; e < ENL_TR * ENL_TC * KT * E; e += ENL_THREADS) V[e] = 0.0;
+    // columns whose window lies inside the image, and the input columns they read
+    const long long cin0 = j0 - hw < 0 ? 0 : j0 - hw;
+    const long long cin1 = j0 + ENL_TC + hw < cols ? j0 + ENL_TC + hw : cols;          // exclusive
+    const long long rin0 = i0 - hw < 0 ? 0 : i0 - hw;
+    const long long rin1 = i0 + ENL_TR + hw < rows ? i0 + ENL_TR + hw : rows;
+    for (long long R = rin0; R < rin1; ++R) {
+        __syncthreads();                                                 // the previous row's H is no longer read
+        for (int e = tid; e < ENL_TC * KT * E; e += ENL_THREADS) H[e] = 0.0;
+        for (long long cs = cin0; cs < cin1; cs += ENL_SEG) {
+            __syncthreads();                                             // S and H free, H zeroed
+            const int nseg = int(cin1 - cs < ENL_SEG ? cin1 - cs : ENL_SEG);
+            for (int q = tid; q < nseg * KT; q += ENL_THREADS) {
+                const int p = q / KT, tt = q - p * KT;
+                double* x = S + q * E;
+                if (t0 + tt < k) {
+                    const T* src = values + R * s0 + (cs + p) * s1 + (long long)(t0 + tt) * s2;
+                    bool finite = true;
+                    for (int b = 0; b < B; ++b) {
+                        x[b] = double(src[b * s3]);
+                        finite = finite && isfinite(x[b]);
+                    }
+                    const double det = sample_det<POL>(x);
+                    x[B] = finite && det > 0.0 ? log(det) : CUDART_NAN;
+                }
+            }
+            __syncthreads();
+            for (int e = tid; e < ENL_TC * KT * E; e += ENL_THREADS) {
+                const int c = e / (KT * E), rest = e - c * (KT * E);
+                const long long j = j0 + c;
+                if (j < hw || j >= cols - hw) continue;                  // border column: no window
+                // this segment's part of the window cols j - hw .. j + hw, left to right
+                const long long a = j - hw > cs ? j - hw : cs;
+                const long long z = j + hw + 1 < cs + nseg ? j + hw + 1 : cs + nseg;
+                double sum = H[e];
+                for (long long jj = a; jj < z; ++jj) sum += S[int(jj - cs) * KT * E + rest];
+                H[e] = sum;
+            }
+        }
+        __syncthreads();
+        // add the row's window sums to the output rows i = i0 + r with |i - R| <= hw (only those rows are touched)
+        const int r0 = R - hw - i0 > 0 ? int(R - hw - i0) : 0;
+        const int r1 = R + hw - i0 < ENL_TR - 1 ? int(R + hw - i0) : ENL_TR - 1;
+        constexpr int ROW = ENL_TC * KT * E;
+        for (int e = r0 * ROW + tid; e < (r1 + 1) * ROW; e += ENL_THREADS) V[e] += H[e % ROW];
+    }
+    __syncthreads();
+    const double N = double(w) * double(w);
+    for (int o = tid; o < ENL_TR * ENL_TC * KT; o += ENL_THREADS) {
+        const int r = o / (ENL_TC * KT), c = (o / KT) % ENL_TC, tt = o % KT;
+        const long long i = i0 + r, j = j0 + c;
+        const int t = t0 + tt;
+        if (i >= rows || j >= cols || t >= k) continue;
+        double out = CUDART_NAN;
+        if (i >= hw && i < rows - hw && j >= hw && j < cols - hw) {
+            const double* v = V + o * E;
+            double M[B];
+#pragma unroll
+            for (int b = 0; b < B; ++b) M[b] = v[b] / N;
+            const double detM = sample_det<POL>(M), delta = log(detM) - v[B] / N;
+            if (!(detM > 0.0) || delta != delta) out = CUDART_NAN;
+            else if (delta <= 0.0) out = CUDART_INF;                     // no speckle
+            else if (delta < CUDART_INF) {
+                constexpr int P = POL == NDCHG_POL_SINGLE ? 1 : POL == NDCHG_POL_DUAL || POL == NDCHG_POL_DUAL_DIAGONAL ? 2 : 3;
+                out = enl_solve<P, POL == NDCHG_POL_SINGLE || POL == NDCHG_POL_DUAL || POL == NDCHG_POL_QUAD>(delta, N);
+            }
+        }
+        enl[(i * cols + j) * k + t] = T(out);
+    }
+}
+
 }  // namespace ndchg
 
 struct ChgDeviceGuard {
@@ -514,6 +698,53 @@ extern "C" int ndchg_change_direction(const void* values, const int64_t shape[3]
     if (rc) return rc;
     return dtype == NDCHG_F64 ? launch_direction<double>(pol, values, shape, strides, result, stream)
                               : launch_direction<float>(pol, values, shape, strides, result, stream);
+}
+
+template <typename T, int POL>
+static int launch_enl(const void* values, const int64_t* shape, const int64_t* strides, uint32_t window, void* enl,
+                      void* stream) {
+    using Tile = ndchg::EnlTile<T, POL>;
+    const dim3 grid(unsigned((shape[2] + Tile::KT - 1) / Tile::KT), unsigned((shape[1] + ndchg::ENL_TC - 1) / ndchg::ENL_TC),
+                    unsigned((shape[0] + ndchg::ENL_TR - 1) / ndchg::ENL_TR));
+    if (grid.y > 65535 || grid.z > 65535) return chg_fail(NDNLM_EINVAL, "image of %lld x %lld pixels is too large for ndchg_enl",
+                                                          (long long)shape[0], (long long)shape[1]);
+    cudaError_t e = cudaFuncSetAttribute(ndchg::enl_kernel<T, POL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Tile::smem));
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "shared memory of %zu bytes: %s", Tile::smem, cudaGetErrorString(e));
+    ndchg::enl_kernel<T, POL><<<grid, ndchg::ENL_THREADS, Tile::smem, (cudaStream_t)stream>>>(
+        (const T*)values, shape[0], shape[1], int(shape[2]), strides[0], strides[1], strides[2], strides[3], int(window), (T*)enl);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+template <typename T>
+static int launch_enl(int pol, const void* values, const int64_t* shape, const int64_t* strides, uint32_t window, void* enl,
+                      void* stream) {
+    switch (pol) {
+        case NDCHG_POL_DUAL: return launch_enl<T, NDCHG_POL_DUAL>(values, shape, strides, window, enl, stream);
+        case NDCHG_POL_SINGLE: return launch_enl<T, NDCHG_POL_SINGLE>(values, shape, strides, window, enl, stream);
+        case NDCHG_POL_QUAD: return launch_enl<T, NDCHG_POL_QUAD>(values, shape, strides, window, enl, stream);
+        case NDCHG_POL_DUAL_DIAGONAL: return launch_enl<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, window, enl, stream);
+        case NDCHG_POL_QUAD_DIAGONAL: return launch_enl<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, window, enl, stream);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+extern "C" int ndchg_enl(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                         uint32_t window, void* enl, void* stream) {
+    if (!values || !shape || !strides || !enl) return chg_fail(NDNLM_EINVAL, "null argument");
+    if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
+    if (pol < NDCHG_POL_DUAL || pol > NDCHG_POL_QUAD_DIAGONAL) return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    if (shape[0] < 1 || shape[1] < 1) return chg_fail(NDNLM_EINVAL, "shape out of range");
+    if (shape[2] < 1 || shape[2] > 0x7fffffffLL) return chg_fail(NDNLM_EINVAL, "the ENL needs at least 1 time step");
+    if (window < 3 || window % 2 == 0) return chg_fail(NDNLM_EINVAL, "the window must be odd and >= 3, got %u", window);
+    if (window > shape[0] || window > shape[1])
+        return chg_fail(NDNLM_EINVAL, "the window (%u) must not exceed the image (%lld x %lld)", window, (long long)shape[0],
+                        (long long)shape[1]);
+    ChgDeviceGuard guard(enl);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "enl is not a CUDA device pointer");
+    return dtype == NDCHG_F64 ? launch_enl<double>(pol, values, shape, strides, window, enl, stream)
+                              : launch_enl<float>(pol, values, shape, strides, window, enl, stream);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }
