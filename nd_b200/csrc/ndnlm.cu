@@ -76,6 +76,7 @@ struct TiledInst {
     int minb;           // CTAs per SM the kernel is compiled for (__launch_bounds__ min blocks)
     bool half;          // the last variable group carries at most two variables (V = 5, 6): its upper lanes are skipped
     bool dh;            // double-duty halo warps (nlm_tiled.cuh, TiledCfg): nwarps warps cover nwarps + fw rows
+    bool persist;       // persistent CTAs (nlm_tiled.cuh, TiledCfg): one W pass, next box loaded during the epilogue
     int nv4, fw, fx, fr, L, nwarps, ch;
     bool neff;
     size_t exch_bytes;
@@ -99,6 +100,9 @@ struct TiledInst {
 #define TILED_INSTD64(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                     \
     extern template cudaError_t launch_tiled<double, NV4, FW, FX, FR, L, NW, CH, NEFF, false, true>(          \
         const CUtensorMap&, const ndnlm::DevParams&, const void*, void*, int*, int, size_t, cudaStream_t);
+#define TILED_INSTP(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                       \
+    extern template cudaError_t launch_tiled<float, NV4, FW, FX, FR, L, NW, CH, NEFF, false, false, true>(   \
+        const CUtensorMap&, const ndnlm::DevParams&, const void*, void*, int*, int, size_t, cudaStream_t);
 #include "instances_g0.inc"
 #include "instances_g1.inc"
 #include "instances_g2.inc"
@@ -106,40 +110,48 @@ struct TiledInst {
 #include "instances_g4.inc"
 #include "instances_g5.inc"
 #include "instances_g6.inc"
+#include "instances_g7.inc"
 #undef TILED_INST
 #undef TILED_INST64
 #undef TILED_INSTH
 #undef TILED_INSTD
 #undef TILED_INSTD64
+#undef TILED_INSTP
 
 #define TILED_INSTD64(NV4, FW, FX, FR, L, NW, CH, NEFF)                                              \
     {                                                                                                \
-        8, 1, false, true, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<double, NV4, FW, FX, FR, L, NW, CH, NEFF, true>::EXCH_BYTES, \
+        8, 1, false, true, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<double, NV4, FW, FX, FR, L, NW, CH, NEFF, true>::EXCH_BYTES, \
             launch_tiled<double, NV4, FW, FX, FR, L, NW, CH, NEFF, false, true>,                     \
             "nlm_tiled<double,nv4=" #NV4 ",f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW "(dh),ch=" #CH ",neff=" #NEFF ">" \
     },
 
 #define TILED_INSTD(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                \
     {                                                                                                \
-        4, 1, false, true, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF, true>::EXCH_BYTES, \
+        4, 1, false, true, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF, true>::EXCH_BYTES, \
             launch_tiled<float, NV4, FW, FX, FR, L, NW, CH, NEFF, false, true>,                      \
             "nlm_tiled<nv4=" #NV4 ",f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW "(dh),ch=" #CH ",neff=" #NEFF ">" \
     },
 #define TILED_INSTH(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                \
     {                                                                                                \
-        4, tiled_min_blocks<float, NV4, FW, L, NW>(), true, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
+        4, tiled_min_blocks<float, NV4, FW, L, NW>(), true, false, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
             launch_tiled<float, NV4, FW, FX, FR, L, NW, CH, NEFF, true>,                             \
             "nlm_tiled<nv4=" #NV4 "(half),f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW ",ch=" #CH ",neff=" #NEFF ">" \
     },
 #define TILED_INST(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                 \
     {                                                                                                \
-        4, tiled_min_blocks<float, NV4, FW, L, NW>(), false, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
+        4, tiled_min_blocks<float, NV4, FW, L, NW>(), false, false, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
             launch_tiled<float, NV4, FW, FX, FR, L, NW, CH, NEFF>,                                   \
             "nlm_tiled<nv4=" #NV4 ",f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW ",ch=" #CH ",neff=" #NEFF ">" \
     },
+#define TILED_INSTP(NV4, FW, FX, FR, L, NW, CH, NEFF)                                                \
+    {                                                                                                \
+        4, 1, false, false, true, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<float, NV4, FW, FX, FR, L, NW, CH, NEFF, false, true>::EXCH_BYTES, \
+            launch_tiled<float, NV4, FW, FX, FR, L, NW, CH, NEFF, false, false, true>,               \
+            "nlm_tiled<nv4=" #NV4 ",f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW "(persist),ch=" #CH ",neff=" #NEFF ">" \
+    },
 #define TILED_INST64(NV4, FW, FX, FR, L, NW, CH, NEFF)                                               \
     {                                                                                                \
-        8, 1, false, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<double, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
+        8, 1, false, false, false, NV4, FW, FX, FR, L, NW, CH, NEFF, TiledCfg<double, NV4, FW, FX, FR, L, NW, CH, NEFF>::EXCH_BYTES, \
             launch_tiled<double, NV4, FW, FX, FR, L, NW, CH, NEFF>,                                  \
             "nlm_tiled<double,nv4=" #NV4 ",f=(" #FW "," #FR "," #FX "),L=" #L ",warps=" #NW ",ch=" #CH ",neff=" #NEFF ">" \
     },
@@ -153,12 +165,14 @@ static const TiledInst g_tiled[] = {
 #include "instances_g4.inc"
 #include "instances_g5.inc"
 #include "instances_g6.inc"
+#include "instances_g7.inc"
 };
 #undef TILED_INST
 #undef TILED_INST64
 #undef TILED_INSTH
 #undef TILED_INSTD
 #undef TILED_INSTD64
+#undef TILED_INSTP
 static const int g_ntiled = int(sizeof(g_tiled) / sizeof(g_tiled[0]));
 
 // ------------------------------------------------------------------------------------------
@@ -223,10 +237,11 @@ static bool configure_tiled(ndnlm_plan* pl, const TiledInst& ti, int elem) {
     const int ntw = 2 * P.rad[0] + 1;
     bool fits = false;
     size_t smem = 0;
-    // kernels compiled for two CTAs per SM first look for a pass count whose box lets two CTAs share the SM's shared memory
+    // kernels compiled for two CTAs per SM first look for a pass count whose box lets two CTAs share the SM's shared memory;
+    // persistent CTAs need the whole W search range in one box
     size_t cap = ti.minb > 1 ? (kMaxSmem / ti.minb - 1024) : kMaxSmem;
     for (int attempt = 0; attempt < 2 && !fits; ++attempt, cap = kMaxSmem)
-    for (int npass = 1; npass <= ntw && !fits; ++npass) {
+    for (int npass = 1; npass <= (ti.persist ? 1 : ntw) && !fits; ++npass) {
         const int per = (ntw + npass - 1) / npass;
         P.npass = (ntw + per - 1) / per;
         P.ntw_pass = per;
@@ -372,17 +387,21 @@ extern "C" int ndnlm_plan_create_roles(ndnlm_plan_t** out_plan, const int64_t sh
     if (kernel != NDNLM_KERNEL_GENERIC && tiled_ok) {
         const char* venv = getenv("NDNLM_TILED_VARIANT");   // tuning aid: force one instantiation
         const int forced = venv ? atoi(venv) : -1;
-        // Two rounds over the table: the double-duty-halo-warp instantiations (instances_g6.inc) first where they are
+        // Three rounds over the table: the double-duty-halo-warp instantiations (instances_g6.inc) first where they are
         // enabled (by default for patch radius f_W >= NDNLM_DH_MIN_FW and for float64; NDNLM_DH=0 / 1 disables /
-        // enables all of them), then everything else in file order.
+        // enables all of them), then the persistent-CTA instantiations (instances_g7.inc; NDNLM_PERSIST=0 disables
+        // them), then everything else in file order.
         const char* denv = getenv("NDNLM_DH");
-        for (int round = 0; round < 2 && pl->inst < 0; ++round) {
+        const char* penv = getenv("NDNLM_PERSIST");
+        const bool use_persist = penv ? atoi(penv) != 0 : true;
+        for (int round = 0; round < 3 && pl->inst < 0; ++round) {
             for (int i = 0; i < g_ntiled; ++i) {
                 if (forced >= 0 && i != forced) continue;
                 // measured (profiles/r2_dh_experiment*.txt): float32 +15 % with four halo rows (f_W = 2), -1 % with two
                 // (f_W = 1: that kernel is bound by the shared-memory pipe, not by latency); float64 +9 % / +24 %
                 const bool use_dh = denv ? atoi(denv) != 0 : (g_tiled[i].fw >= NDNLM_DH_MIN_FW || g_tiled[i].elem == 8);
-                if (forced < 0 && (g_tiled[i].dh != (round == 0) || (g_tiled[i].dh && !use_dh))) continue;
+                const int group = g_tiled[i].dh ? 0 : g_tiled[i].persist ? 1 : 2;
+                if (forced < 0 && (group != round || (g_tiled[i].dh && !use_dh) || (g_tiled[i].persist && !use_persist))) continue;
                 if (configure_tiled(pl, g_tiled[i], elem)) {
                     pl->kernel = NDNLM_KERNEL_TILED;
                     pl->inst = i;
@@ -676,6 +695,18 @@ static encode_tiled_fn get_encode_fn() {
     return fn;
 }
 
+#if NDNLM_TILE_PROBE
+// Development builds only (-DNDNLM_TILE_PROBE=1, tools/dev_tile_probe.py): the device buffer of [tile][8] uint64 the next
+// tiled-kernel launches record their tile timelines into; cap = 0 stops recording.
+static unsigned long long* g_probe = nullptr;
+static int g_probe_cap = 0;
+extern "C" int ndnlm_tile_probe(void* buf, int cap) {
+    g_probe = static_cast<unsigned long long*>(buf);
+    g_probe_cap = buf ? cap : 0;
+    return NDNLM_OK;
+}
+#endif
+
 extern "C" size_t ndnlm_scratch_bytes(const ndnlm_plan_t* pl) {
     if (!pl || !pl->boxmean) return 0;
     const DevParams& P = pl->P;
@@ -719,7 +750,14 @@ extern "C" int ndnlm_run_scratch(const ndnlm_plan_t* pl, const void* padded, voi
                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
             if (cr != CUDA_SUCCESS) return fail(NDNLM_ECUDA, "cuTensorMapEncodeTiled failed with CUresult %d", int(cr));
         }
+#if NDNLM_TILE_PROBE
+        DevParams PP = P;
+        PP.probe = g_probe;
+        PP.probe_cap = g_probe_cap;
+        cudaError_t e = ti.launch(tmap, PP, padded, out_internal, err_flag, pl->grid, pl->smem, st);
+#else
         cudaError_t e = ti.launch(tmap, P, padded, out_internal, err_flag, pl->grid, pl->smem, st);
+#endif
         g_launches++;
         if (e != cudaSuccess) return fail(NDNLM_ECUDA, "tiled kernel launch failed: %s", cudaGetErrorString(e));
     } else if (pl->dtype == NDNLM_F64) {

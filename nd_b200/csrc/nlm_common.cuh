@@ -12,6 +12,11 @@
 #include <cuda.h>
 #include <stdint.h>
 
+#ifndef NDNLM_TILE_PROBE
+#define NDNLM_TILE_PROBE 0   // 1 (development): one warp of the tiled kernel records clock64() at the phase boundaries of
+                             //    every tile into DevParams::probe (tools/dev_tile_probe.py)
+#endif
+
 #ifndef __CUDA_ARCH__
 #define NDNLM_HOST_SIDE 1
 #endif
@@ -44,6 +49,10 @@ struct DevParams {
     double n_eff;      // < 0: self weight = max weight  (:406-413)
     int zero_dist;     // reference_compiled semantics with some f_i > 0 (SURVEY F1)
     int use_ldg_loader;// debugging: fill the tile with plain loads instead of TMA
+#if NDNLM_TILE_PROBE
+    unsigned long long* probe;   // [tile][8]: clock64() at the tile's phase boundaries, slot 7 the SM id
+    int probe_cap;               // tiles the buffer holds
+#endif
 };
 
 __host__ __device__ inline int reflect_index(int i, int n) {

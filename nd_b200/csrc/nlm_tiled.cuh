@@ -250,14 +250,19 @@ __device__ __forceinline__ P2 lane_box_sum2(const P2 v) {
 // row they leave their warp scheduler under-used and occupy 2 FW of the NWARPS register-file slots.  With DH each of FW
 // halo WARPS serves TWO halo rows (one above, one below the valid rows; it keeps no accumulators, so the second centre
 // column fits its registers): NWARPS warps then cover NWARPS + FW rows, NWARPS - FW of them valid.
-template <typename T, int NV4, int FW, int FX, int FR, int L, int NWARPS, int CH, bool NEFF, bool DH = false>
+// PERSIST: persistent CTAs (one per SM) that walk tiles blockIdx.x + k gridDim.x, keep the whole W search range in
+// shared memory (one pass), read the centre column from it and load the next tile's box while the finished tile runs its
+// epilogue.  The W exchange then only holds the TXW valid lanes of a row: the sums of the X-halo lanes are never read.
+template <typename T, int NV4, int FW, int FX, int FR, int L, int NWARPS, int CH, bool NEFF, bool DH = false,
+          bool PERSIST = false>
 struct TiledCfg {
     static constexpr int E = L + 2 * FR;      // column elements including the patch halo
     static constexpr int WN = E + CH - 1;     // neighbour window elements per chunk of CH R-offsets
     static constexpr int TXW = 32 - 2 * FX;   // valid lanes per warp
     static constexpr int THREADS = NWARPS * 32;
     static constexpr int NROWS = DH ? NWARPS + FW : NWARPS;   // W rows of the CTA tile, patch-halo rows included
-    static constexpr size_t EXCH_BYTES = FW > 0 ? size_t(CH) * NROWS * (L / 2) * 32 * sizeof(typename Elem<T>::P2) : 0;
+    static constexpr int EXW = PERSIST ? TXW : 32;             // exchange slots per row and R-offset
+    static constexpr size_t EXCH_BYTES = FW > 0 ? size_t(CH) * NROWS * (L / 2) * EXW * sizeof(typename Elem<T>::P2) : 0;
 };
 
 // HALF: the last variable group holds at most two real variables (V = 5 or 6 of 8): its upper two lanes are zero
@@ -271,17 +276,19 @@ constexpr int tiled_min_blocks() {
     return (sizeof(T) == 4 && NV4 == 1 && L <= 4 && NWARPS <= 4) ? 4 : (sizeof(T) == 4 && NV4 == 1 && L <= 4 && NWARPS <= 8) ? 2 : 1;
 }
 
-template <typename T, int NV4, int FW, int FX, int FR, int L, int NWARPS, int CH, bool NEFF, bool HALF = false, bool DH = false>
+template <typename T, int NV4, int FW, int FX, int FR, int L, int NWARPS, int CH, bool NEFF, bool HALF = false, bool DH = false,
+          bool PERSIST = false>
 __global__ void __launch_bounds__(NWARPS * 32, tiled_min_blocks<T, NV4, FW, L, NWARPS>())
 nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
                  const typename Elem<T>::V4* __restrict__ padded, typename Elem<T>::V4* __restrict__ out,
                  int* __restrict__ err) {
-    using Cfg = TiledCfg<T, NV4, FW, FX, FR, L, NWARPS, CH, NEFF, DH>;
+    using Cfg = TiledCfg<T, NV4, FW, FX, FR, L, NWARPS, CH, NEFF, DH, PERSIST>;
     using V4 = typename Elem<T>::V4;
     using P2 = typename Elem<T>::P2;
     constexpr bool F64 = sizeof(T) == 8;
     static_assert(L % 2 == 0, "L must be even (outputs are exchanged in pairs)");
     static_assert(!DH || (FW > 0 && NWARPS >= 3 * FW + 1), "double-duty halo warps need a W patch axis");
+    static_assert(!PERSIST || (!F64 && !HALF && !DH && FW > 0 && L == 4), "persistent CTAs: float32, L = 4, W patch axis");
     constexpr int E = Cfg::E, TXW = Cfg::TXW;
     constexpr int NROWS = Cfg::NROWS;                      // W rows of the tile (== NWARPS unless DH)
 
@@ -302,14 +309,35 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
     uint64_t* mbar_full = mbar + 1;
     uint64_t* mbar_empty = mbar + 1 + NROWS;
 
-    int bid = blockIdx.x;
+    // PERSIST: this CTA's tk-th tile is tile_id = blockIdx.x + tk gridDim.x, in the order of the one-tile-per-CTA launch
+    [[maybe_unused]] const int ntiles = P.tiles[0] * P.tiles[1] * P.tiles[2];
+    [[maybe_unused]] int tile_id = blockIdx.x, tk = 0;
+    [[maybe_unused]] uint32_t xpar_carry = 0;   // exchange parity at the end of the previous tile
+#if NDNLM_TILE_PROBE
+#define NDNLM_PROBE(slot)                                                                         \
+    do {                                                                                          \
+        if (threadIdx.x == 32 * FW && tile_id < P.probe_cap) P.probe[size_t(tile_id) * 8 + (slot)] = clock64(); \
+    } while (0)
+#else
+#define NDNLM_PROBE(slot) do {} while (0)
+#endif
+    do {
+    NDNLM_PROBE(0);
+    int bid = PERSIST ? tile_id : int(blockIdx.x);
     const int tileX = bid % P.tiles[2];
     bid /= P.tiles[2];
     const int tileR = bid % P.tiles[1];
     const int tileW = bid / P.tiles[1];
     const int w0 = tileW * P.t[0], r0 = tileR * P.t[1], x0 = tileX * P.t[2];
-
+#if NDNLM_TILE_PROBE
+    if (threadIdx.x == 32 * FW && tile_id < P.probe_cap) {
+        unsigned sm;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
+        P.probe[size_t(tile_id) * 8 + 7] = sm;
+    }
+#endif
     // ---- stage the padded box (tile + halo r+f) into shared memory ----
+    if (!PERSIST || tk == 0) {
     if (threadIdx.x == 0) {
         mbar_init(mbar, 1);
         if constexpr (FW > 0) {
@@ -327,6 +355,7 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
         fence_mbar_init();
     }
     __syncthreads();
+    }
     // The W search range [-rW, rW] is covered in P.npass passes of P.ntw_pass offsets each; a pass keeps
     // only the rows it needs in shared memory (BW = rows of the CTA + ntw_pass - 1), which is what lets
     // more warps fit beside the exchange buffer.  Pass `p` starts at padded row w0 + p * ntw_pass.
@@ -371,9 +400,9 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
     const bool wvalid = (FW == 0) || (ww >= FW && ww < NROWS - FW);
     const int xw = DH ? ww : wid;                          // my row's index among the exchange slots / mbarriers
 
-    // centre column: read once, straight from the padded cube (R is the fastest axis there too)
+    // centre column: read once, straight from the padded cube (R is the fastest axis there too); PERSIST: from the box
     V4 c[NV4][E];
-    {
+    if constexpr (!PERSIST) {
         const int gw = w0 + ww + P.rad[0], gx = x0 + lx;      // padded coordinates of this thread's column
         const bool inb = gw < P.pd[0] && gx < P.pd[2];
 #pragma unroll
@@ -430,9 +459,14 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
     P2* const ex_own = exch + (xw * (L / 2)) * 32 + lane;     // + (j*NWARPS*(L/2) + o2)*32
     constexpr int EX_J = NROWS * (L / 2) * 32;                      // float2 stride between R-offsets j
     constexpr int EX_ROW = (L / 2) * 32;                            // float2 stride between W rows (FW>0: 1 warp/row)
-    [[maybe_unused]] V4* const ex_own4 = reinterpret_cast<V4*>(exch) + xw * 32 + lane;   // L == 4 layout
-    [[maybe_unused]] constexpr int EX_J4 = NROWS * 32;              // float4 stride between R-offsets j
-    uint32_t xpar = 0;                                              // parity of the current exchange round
+    // L == 4 layout [j][row][slot] float4.  PERSIST: slots are the valid lanes only; the X-halo lanes store nothing and read
+    // their neighbour's slot (their sums, weights and accumulators are never used)
+    constexpr int EXW = Cfg::EXW;
+    [[maybe_unused]] V4* const ex_own4 =
+        reinterpret_cast<V4*>(exch) + xw * EXW + (PERSIST ? min(max(lane - FX, 0), TXW - 1) : lane);
+    [[maybe_unused]] constexpr int EX_J4 = NROWS * EXW;             // float4 stride between R-offsets j
+    [[maybe_unused]] const bool ex_store = !PERSIST || (lane >= FX && lane < 32 - FX);
+    uint32_t xpar = PERSIST ? xpar_carry : 0;                       // parity of the current exchange round
     static_assert(FW == 0 || NROWS >= 2 * FW + 2, "every row needs at least one reader");
 
     // One chunk of NJ consecutive R-offsets [ch0, ch0+NJ).  NJ is a compile-time constant so the body is
@@ -539,7 +573,7 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
                 }
                 if constexpr (L == 4) {
                     // one 16-B store / load per row and offset: [j][row][lane] float4
-                    ex_own4[j * EX_J4] = mk4(px[0].x, px[0].y, px[1].x, px[1].y);
+                    if (ex_store) ex_own4[j * EX_J4] = mk4(px[0].x, px[0].y, px[1].x, px[1].y);
                 } else {
 #pragma unroll
                     for (int o2 = 0; o2 < L / 2; ++o2) ex_own[j * EX_J + o2 * 32] = px[o2];
@@ -569,7 +603,7 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
                     }
                     P2 D[L / 2];
                     if constexpr (L == 4) {
-                        V4 t = ex_own4[j * EX_J4 - FW * 32];
+                        V4 t = ex_own4[j * EX_J4 - FW * EXW];
                         D[0] = mk2(t.x, t.y);
                         D[1] = mk2(t.z, t.w);
 #pragma unroll
@@ -578,7 +612,7 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
                                 D[0] = padd(D[0], own[j][0]);
                                 D[1] = padd(D[1], own[j][1]);
                             } else {
-                                t = ex_own4[j * EX_J4 + d * 32];
+                                t = ex_own4[j * EX_J4 + d * EXW];
                                 D[0] = padd(D[0], mk2(t.x, t.y));
                                 D[1] = padd(D[1], mk2(t.z, t.w));
                             }
@@ -729,11 +763,30 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
             return;
         }
     }
-    for (int pass = 0; pass < P.npass; ++pass) {
+    for (int pass = 0; pass < (PERSIST ? 1 : P.npass); ++pass) {
         const int twa = -rW + pass * P.ntw_pass;
         const int twb = min(rW, twa + P.ntw_pass - 1);
-        if (pass > 0) __syncthreads();     // every warp is done with the previous pass's rows
-        load_pass(pass);
+        if (pass > 0) {                    // every warp is done with the previous pass's rows
+            NDNLM_PROBE(2);
+            __syncthreads();
+            NDNLM_PROBE(3);
+        }
+        if constexpr (PERSIST) {
+            // the box of every tile but the first was requested at the end of the previous tile
+            if (tk > 0 && !P.use_ldg_loader) mbar_wait(mbar, uint32_t(tk & 1));
+            else load_pass(0);
+        } else {
+            load_pass(pass);
+        }
+        NDNLM_PROBE(pass == 0 ? 1 : 4);
+        if constexpr (PERSIST) {
+            // one pass: every row of the tile, halo rows included, is in the box (padded row w0 + ww + rW is box row ww + rW)
+            const V4* cs = tile + ((ww + rW) * BX + lx) * BRP + lr0;
+#pragma unroll
+            for (int q = 0; q < NV4; ++q)
+#pragma unroll
+                for (int e = 0; e < E; ++e) c[q][e] = cs[size_t(q) * plane + e];
+        }
         if (nR <= CH) {
             dispatch_chunk<CH>(nR, false, [&](auto nj_tag, auto) {
                 for (int tw = twa; tw <= twb; ++tw) {
@@ -760,6 +813,25 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
                 }
                 fold_weight_sums();
             }
+        }
+    }
+
+    NDNLM_PROBE(5);
+    if constexpr (PERSIST) {
+        // The box is dead once every warp is here: request the next tile's box now, so that it lands while this tile runs
+        // its epilogue (registers and global memory only).  Every exchange round of this tile is complete as well.
+        __syncthreads();
+        NDNLM_PROBE(3);
+        xpar_carry = xpar;
+        const int next = tile_id + int(gridDim.x);
+        if (threadIdx.x == 0 && next < ntiles && !P.use_ldg_loader) {
+            int nb = next;
+            const int nx0 = (nb % P.tiles[2]) * P.t[2];
+            nb /= P.tiles[2];
+            const int nr0 = (nb % P.tiles[1]) * P.t[1], nw0 = (nb / P.tiles[1]) * P.t[0];
+            mbar_arrive_expect_tx(mbar, uint32_t(NV4) * uint32_t(BW * BRP * BX) * uint32_t(sizeof(V4)));
+#pragma unroll
+            for (int q = 0; q < NV4; ++q) tma_load_5d(tile + size_t(q) * plane, &tmap, mbar, 0, nr0, nx0, nw0, q);
         }
     }
 
@@ -814,6 +886,14 @@ nlm_tiled_kernel(const __grid_constant__ CUtensorMap tmap, const DevParams P,
             }
         }
     }
+#if NDNLM_TILE_PROBE
+    __syncwarp();
+#endif
+    NDNLM_PROBE(6);
+    tile_id += int(gridDim.x);
+    ++tk;
+    } while (PERSIST && tile_id < ntiles);
+#undef NDNLM_PROBE
 }
 
 }  // namespace ndnlm
