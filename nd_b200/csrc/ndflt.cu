@@ -554,20 +554,22 @@ static bool try_rows_smem(const TileGeom& TG, const void* in, void* out, const d
     RG.mode = TG.mode;
     RG.cval = TG.cval;
     const size_t smem = size_t(RG.LN) * RG.pitch * 8 + size_t(nw) * 8;
-    if (SYM != 0 && size1 == size2 && size1 >= 1 && size1 <= 8) {
-        switch (size1) {
-            case 1: launch_rows_smem<T, SYM, 1>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 2: launch_rows_smem<T, SYM, 2>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 3: launch_rows_smem<T, SYM, 3>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 4: launch_rows_smem<T, SYM, 4>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 5: launch_rows_smem<T, SYM, 5>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 6: launch_rows_smem<T, SYM, 6>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            case 7: launch_rows_smem<T, SYM, 7>(RG, smem, in, out, dw, size1, size2, origin, st); break;
-            default: launch_rows_smem<T, SYM, 8>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+    if constexpr (SYM != 0) {                                        // general kernels only take the S1 = 0 form
+        if (size1 == size2 && size1 >= 1 && size1 <= 8) {
+            switch (size1) {
+                case 1: launch_rows_smem<T, SYM, 1>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 2: launch_rows_smem<T, SYM, 2>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 3: launch_rows_smem<T, SYM, 3>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 4: launch_rows_smem<T, SYM, 4>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 5: launch_rows_smem<T, SYM, 5>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 6: launch_rows_smem<T, SYM, 6>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                case 7: launch_rows_smem<T, SYM, 7>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+                default: launch_rows_smem<T, SYM, 8>(RG, smem, in, out, dw, size1, size2, origin, st); break;
+            }
+            return true;
         }
-    } else {
-        launch_rows_smem<T, SYM, 0>(RG, smem, in, out, dw, size1, size2, origin, st);
     }
+    launch_rows_smem<T, SYM, 0>(RG, smem, in, out, dw, size1, size2, origin, st);
     return true;
 }
 
