@@ -114,6 +114,36 @@ int ndchg_change_direction(const void* values, const int64_t shape[3], const int
 int ndchg_enl(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol, uint32_t window,
               void* enl, void* stream);
 
+/* Refined Lee speckle filter (Lee, Grunes & de Grandi, IEEE TGRS 37(5), 1999) of every time step on its own, over
+ * an N x N window, N = `window` in {7, 11, 15} (N = 4m + 3; 7 is Lee et al.'s), N <= min(rows, cols); `looks` L
+ * is finite and > 0.  `values` as above, in the band order of `pol`; `out` is a DEVICE array (rows, cols, k,
+ * bands) of the data type, C-contiguous, written completely, not overlapping `values`.  Requires k >= 1.
+ *
+ * h = N / 2, subwindow side s = (N - 1) / 2 (odd), subwindow spacing c = (N - s) / 2 (N = 7: s = 3, c = 2).  Samples
+ * outside the image are scipy's 'reflect' (half-sample symmetric) images of samples inside, one reflection deep.
+ * For every output pixel p, over the offsets (dy, dx) in [-h, h]^2 of its window:
+ *   1. span y = the diagonal bands added left to right, C11 + C22 (+ C33); single-pol: C11.
+ *   2. m[u][v], u, v in {0, 1, 2}: the mean of y over the s x s subwindow centred at ((u - 1) c, (v - 1) c),
+ *      summed row-major, divided by s^2.
+ *   3. G0 = |(m02 + m12 + m22) - (m00 + m10 + m20)|,  G1 = |(m20 + m21 + m22) - (m00 + m01 + m02)|,
+ *      G2 = |(m01 + m02 + m12) - (m10 + m20 + m21)|,  G3 = |(m00 + m01 + m10) - (m12 + m21 + m22)|  (each
+ *      three-term sum added left to right); e = 0, then e = i for i = 1, 2, 3 if Gi > Ge (the first maximum
+ *      wins; NaN never wins).
+ *   4. (first, second) = (m10, m12), (m01, m21), (m02, m20), (m00, m22) for e = 0 .. 3, with the masks
+ *      d <= 0 / d >= 0 of d = dx, dy, dy - dx, dy + dx; the second mask iff |second - m11| < |first - m11|.
+ *      A mask holds n = N (N + 1) / 2 offsets.
+ *   5. over the mask, row-major (dy outer, dx inner, both ascending): ybar = sum y / n,
+ *      var_y = sum (y - ybar)(y - ybar) / n, sv2 = 1 / L, var_x = (var_y - (ybar ybar) sv2) / (1 + sv2),
+ *      b = var_x > 0 ? var_x / var_y : 0.
+ *   6. every band: M = (sum over the mask, row-major) / n, out = M + b (x_p - M).
+ * Arithmetic: inputs are read in the data type; everything else is one correctly rounded double operation at a
+ * time (no FMA contraction); every sum is a direct sum in the order given (acc = acc + term from acc = 0, never a
+ * running add / subtract); the result is rounded once to the data type.  NaN follows the arithmetic.  Since
+ * 0 <= b < 1, every output is a convex combination of the sample and a local mean: positive semidefinite samples
+ * stay positive semidefinite. */
+int ndchg_refined_lee(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                      uint32_t window, double looks, void* out, void* stream);
+
 const char* ndchg_last_error(void);
 
 #ifdef __cplusplus

@@ -33,7 +33,8 @@ SYMBOLS = [
 FLT_SYMBOLS = ["ndflt_correlate", "ndflt_correlate1d", "ndflt_launch_count", "ndflt_last_error"]
 # every symbol include/ndchg.h declares (omnibus change detection, SURVEY.md 8(f) row N4)
 CHG_SYMBOLS = ["ndchg_change_detection", "ndchg_omnibus_probability", "ndchg_change_detection_pol",
-               "ndchg_omnibus_probability_pol", "ndchg_change_direction", "ndchg_enl", "ndchg_last_error"]
+               "ndchg_omnibus_probability_pol", "ndchg_change_direction", "ndchg_enl", "ndchg_refined_lee",
+               "ndchg_last_error"]
 
 
 class Info(ctypes.Structure):
@@ -141,6 +142,8 @@ def lib():
     L.ndchg_change_direction.restype = ctypes.c_int
     L.ndchg_enl.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, vp, vp]
     L.ndchg_enl.restype = ctypes.c_int
+    L.ndchg_refined_lee.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, ctypes.c_double, vp, vp]
+    L.ndchg_refined_lee.restype = ctypes.c_int
     L.ndchg_last_error.argtypes = []
     L.ndchg_last_error.restype = ctypes.c_char_p
     _lib = L

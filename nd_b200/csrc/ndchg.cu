@@ -10,6 +10,7 @@
 #include "../../include/ndchg.h"
 #include "../../include/ndnlm.h"
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 
@@ -544,6 +545,138 @@ enl_kernel(const T* __restrict__ values, const long long rows, const long long c
     }
 }
 
+// ---- refined Lee filter (ndchg_refined_lee, include/ndchg.h) ------------------------------------------------------
+// One CTA: a LEE_T x LEE_T tile of output pixels of one time step, one thread per pixel.  The time step is
+// blockIdx.x, so the CTAs of neighbouring steps, which read the same pixel records, run close together.  The
+// (LEE_T + N - 1)^2 input samples of the tile and its halo are staged in shared memory in double, band-planar, with
+// the span as plane B; then the s x s box mean of the span at each of the (LEE_T + 2c)^2 subwindow centres the tile
+// uses is formed once (nine output pixels read each).  Each thread then selects its mask and forms its masked sums
+// over the whole N x N window, adding only the offsets inside the mask: all threads of a warp read the same offset
+// at the same time, so the shared-memory reads stay conflict-free whichever masks the threads chose.
+constexpr int LEE_T = 16, LEE_THREADS = LEE_T * LEE_T;
+
+// number of diagonal bands of a layout, and the band of the d-th one
+__host__ __device__ constexpr int lee_diagonals(const int pol) {
+    return pol == NDCHG_POL_SINGLE ? 1 : pol == NDCHG_POL_DUAL || pol == NDCHG_POL_DUAL_DIAGONAL ? 2 : 3;
+}
+__host__ __device__ constexpr int lee_diagonal_band(const int pol, const int d) {
+    return pol == NDCHG_POL_DUAL ? 3 * d : pol == NDCHG_POL_QUAD ? (d == 0 ? 0 : d == 1 ? 5 : 8) : d;
+}
+
+__host__ __device__ constexpr size_t lee_smem(const int bands, const int N) {
+    return sizeof(double) * (size_t(bands + 1) * (LEE_T + N - 1) * (LEE_T + N - 1) +
+                             size_t(LEE_T + N - (N - 1) / 2) * (LEE_T + N - (N - 1) / 2));
+}
+
+// scipy's 'reflect' (half-sample symmetric) index, one reflection deep; clamped so that the staged positions no
+// output reads (beyond the last tile's pixels) stay inside the image
+__device__ __forceinline__ long long lee_reflect(long long r, const long long n) {
+    r = r < 0 ? -r - 1 : r >= n ? 2 * n - 1 - r : r;
+    return r < 0 ? 0 : r >= n ? n - 1 : r;
+}
+
+__device__ __forceinline__ double add3_(const double a, const double b, const double c) { return add_(add_(a, b), c); }
+
+template <typename T, int POL>
+__global__ void __launch_bounds__(LEE_THREADS)
+refined_lee_kernel(const T* __restrict__ values, const long long rows, const long long cols, const int k,
+                   const long long s0, const long long s1, const long long s2, const long long s3, const int N,
+                   const double looks, T* __restrict__ out) {
+    constexpr int B = pol_bands(POL), P = lee_diagonals(POL);
+    const int h = N / 2, s = (N - 1) / 2, c = (N - s) / 2;
+    const int S = LEE_T + N - 1, BX = LEE_T + 2 * c;
+    extern __shared__ double smem[];
+    double* X = smem;                                                    // [B + 1][S][S]: the bands, then the span
+    double* Y = X + B * S * S;
+    double* box = Y + S * S;                                             // [BX][BX]
+    const int tid = threadIdx.x, t = blockIdx.x;
+    const long long i0 = (long long)blockIdx.z * LEE_T, j0 = (long long)blockIdx.y * LEE_T;
+    for (int q = tid; q < S * S; q += LEE_THREADS) {
+        const int a = q / S, b = q - a * S;
+        const T* src = values + lee_reflect(i0 - h + a, rows) * s0 + lee_reflect(j0 - h + b, cols) * s1 + (long long)t * s2;
+        double x[B];
+#pragma unroll
+        for (int band = 0; band < B; ++band) {
+            x[band] = double(src[band * s3]);
+            X[band * S * S + q] = x[band];
+        }
+        double y = x[lee_diagonal_band(POL, 0)];
+#pragma unroll
+        for (int d = 1; d < P; ++d) y = add_(y, x[lee_diagonal_band(POL, d)]);
+        Y[q] = y;
+    }
+    __syncthreads();
+    // box[p][q]: the mean of the span over staged rows p .. p + s - 1, columns q .. q + s - 1, i.e. the subwindow
+    // centred at staged (p + h - c, q + h - c), since c + (s - 1) / 2 = h
+    const double ss = double(s * s);
+    for (int q = tid; q < BX * BX; q += LEE_THREADS) {
+        const int a = q / BX, b = q - a * BX;
+        double acc = 0.0;
+        for (int u = 0; u < s; ++u)
+            for (int v = 0; v < s; ++v) acc = add_(acc, Y[(a + u) * S + b + v]);
+        box[q] = __ddiv_rn(acc, ss);
+    }
+    __syncthreads();
+    const int ty = tid / LEE_T, tx = tid - ty * LEE_T;
+    const long long i = i0 + ty, j = j0 + tx;
+    if (i >= rows || j >= cols) return;
+    // pixel (ty, tx) is staged at (ty + h, tx + h); its subwindow (u, v) is box[ty + u c][tx + v c]
+    const double* mb = box + ty * BX + tx;
+    const double m00 = mb[0], m01 = mb[c], m02 = mb[2 * c];
+    const double m10 = mb[c * BX], m11 = mb[c * BX + c], m12 = mb[c * BX + 2 * c];
+    const double m20 = mb[2 * c * BX], m21 = mb[2 * c * BX + c], m22 = mb[2 * c * BX + 2 * c];
+    const double G0 = fabs(sub_(add3_(m02, m12, m22), add3_(m00, m10, m20)));
+    const double G1 = fabs(sub_(add3_(m20, m21, m22), add3_(m00, m01, m02)));
+    const double G2 = fabs(sub_(add3_(m01, m02, m12), add3_(m10, m20, m21)));
+    const double G3 = fabs(sub_(add3_(m00, m01, m10), add3_(m12, m21, m22)));
+    int e = 0;
+    double Ge = G0;
+    if (G1 > Ge) { e = 1; Ge = G1; }
+    if (G2 > Ge) { e = 2; Ge = G2; }
+    if (G3 > Ge) e = 3;
+    const double first = e == 0 ? m10 : e == 1 ? m01 : e == 2 ? m02 : m00;
+    const double second = e == 0 ? m12 : e == 1 ? m21 : e == 2 ? m20 : m22;
+    // the mask is sg * (ay dy + ax dx) <= 0
+    const int sg = fabs(sub_(second, m11)) < fabs(sub_(first, m11)) ? -1 : 1;
+    const int ay = e == 0 ? 0 : sg, ax = e == 0 ? sg : e == 1 ? 0 : e == 2 ? -sg : sg;
+    const double* Yw = Y + ty * S + tx;                                  // the window's top-left sample
+    double sy = 0.0;
+    for (int dy = 0; dy < N; ++dy)
+        for (int dx = 0; dx < N; ++dx) {
+            const double v = add_(sy, Yw[dy * S + dx]);
+            sy = ay * (dy - h) + ax * (dx - h) <= 0 ? v : sy;
+        }
+    const double n = double(N * (N + 1) / 2);
+    const double ybar = __ddiv_rn(sy, n);
+    double vy = 0.0, sx[B];
+#pragma unroll
+    for (int band = 0; band < B; ++band) sx[band] = 0.0;
+    for (int dy = 0; dy < N; ++dy)
+        for (int dx = 0; dx < N; ++dx) {
+            const bool in = ay * (dy - h) + ax * (dx - h) <= 0;
+            const int o = dy * S + dx;
+            const double dv = sub_(Yw[o], ybar);
+            const double v = add_(vy, mul_(dv, dv));
+            vy = in ? v : vy;
+#pragma unroll
+            for (int band = 0; band < B; ++band) {
+                const double w = add_(sx[band], Yw[o + (band - B) * S * S]);
+                sx[band] = in ? w : sx[band];
+            }
+        }
+    const double var_y = __ddiv_rn(vy, n);
+    const double sv2 = __ddiv_rn(1.0, looks);
+    const double var_x = __ddiv_rn(sub_(var_y, mul_(mul_(ybar, ybar), sv2)), add_(1.0, sv2));
+    const double wgt = var_x > 0.0 ? __ddiv_rn(var_x, var_y) : 0.0;
+    T* o = out + ((i * cols + j) * k + t) * B;
+    const int centre = (h * S + h) - B * S * S;                          // the pixel's own sample, band 0, from Yw
+#pragma unroll
+    for (int band = 0; band < B; ++band) {
+        const double M = __ddiv_rn(sx[band], n);
+        o[band] = T(add_(M, mul_(wgt, sub_(Yw[centre + band * S * S], M))));
+    }
+}
+
 }  // namespace ndchg
 
 struct ChgDeviceGuard {
@@ -745,6 +878,77 @@ extern "C" int ndchg_enl(const void* values, const int64_t shape[3], const int64
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "enl is not a CUDA device pointer");
     return dtype == NDCHG_F64 ? launch_enl<double>(pol, values, shape, strides, window, enl, stream)
                               : launch_enl<float>(pol, values, shape, strides, window, enl, stream);
+}
+
+template <typename T, int POL>
+static int launch_refined_lee(const void* values, const int64_t* shape, const int64_t* strides, uint32_t window,
+                              double looks, void* out, void* stream) {
+    const dim3 grid(unsigned(shape[2]), unsigned((shape[1] + ndchg::LEE_T - 1) / ndchg::LEE_T),
+                    unsigned((shape[0] + ndchg::LEE_T - 1) / ndchg::LEE_T));
+    if (grid.y > 65535 || grid.z > 65535)
+        return chg_fail(NDNLM_EINVAL, "image of %lld x %lld pixels is too large for ndchg_refined_lee", (long long)shape[0],
+                        (long long)shape[1]);
+    const size_t smem = ndchg::lee_smem(ndchg::pol_bands(POL), int(window));
+    cudaError_t e = cudaFuncSetAttribute(ndchg::refined_lee_kernel<T, POL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "shared memory of %zu bytes: %s", smem, cudaGetErrorString(e));
+    ndchg::refined_lee_kernel<T, POL><<<grid, ndchg::LEE_THREADS, smem, (cudaStream_t)stream>>>(
+        (const T*)values, shape[0], shape[1], int(shape[2]), strides[0], strides[1], strides[2], strides[3], int(window),
+        looks, (T*)out);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+template <typename T>
+static int launch_refined_lee(int pol, const void* values, const int64_t* shape, const int64_t* strides, uint32_t window,
+                              double looks, void* out, void* stream) {
+    switch (pol) {
+        case NDCHG_POL_DUAL: return launch_refined_lee<T, NDCHG_POL_DUAL>(values, shape, strides, window, looks, out, stream);
+        case NDCHG_POL_SINGLE: return launch_refined_lee<T, NDCHG_POL_SINGLE>(values, shape, strides, window, looks, out, stream);
+        case NDCHG_POL_QUAD: return launch_refined_lee<T, NDCHG_POL_QUAD>(values, shape, strides, window, looks, out, stream);
+        case NDCHG_POL_DUAL_DIAGONAL:
+            return launch_refined_lee<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, window, looks, out, stream);
+        case NDCHG_POL_QUAD_DIAGONAL:
+            return launch_refined_lee<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, window, looks, out, stream);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+// true if the bytes `values` spans (any strides, including negative ones) meet the C-contiguous output
+static bool lee_overlap(const void* values, const int64_t* shape, const int64_t* strides, int bands, size_t elem, const void* out) {
+    const int64_t n[4] = {shape[0], shape[1], shape[2], bands};
+    const char* lo = (const char*)values;
+    const char* hi = lo + elem;
+    for (int d = 0; d < 4; ++d) {
+        const int64_t ext = (n[d] - 1) * strides[d] * int64_t(elem);
+        if (ext < 0) lo += ext;
+        else hi += ext;
+    }
+    const char* olo = (const char*)out;
+    const char* ohi = olo + shape[0] * shape[1] * shape[2] * bands * int64_t(elem);
+    return lo < ohi && olo < hi;
+}
+
+extern "C" int ndchg_refined_lee(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                                 uint32_t window, double looks, void* out, void* stream) {
+    if (!values || !shape || !strides || !out) return chg_fail(NDNLM_EINVAL, "null argument");
+    if (pol < NDCHG_POL_DUAL || pol > NDCHG_POL_QUAD_DIAGONAL) return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    if (window != 7 && window != 11 && window != 15)
+        return chg_fail(NDNLM_EINVAL, "the window must be 7, 11 or 15 (4 m + 3), got %u", window);
+    if (shape[0] < 1 || shape[1] < 1) return chg_fail(NDNLM_EINVAL, "shape out of range");
+    if (window > shape[0] || window > shape[1])
+        return chg_fail(NDNLM_EINVAL, "the window (%u) must not exceed the image (%lld x %lld)", window, (long long)shape[0],
+                        (long long)shape[1]);
+    if (shape[2] < 1 || shape[2] > 0x7fffffffLL) return chg_fail(NDNLM_EINVAL, "the refined Lee filter needs at least 1 time step");
+    if (!(looks > 0.0) || !std::isfinite(looks))
+        return chg_fail(NDNLM_EINVAL, "the number of looks must be finite and > 0, got %g", looks);
+    if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out))
+        return chg_fail(NDNLM_EINVAL, "out must not overlap values");
+    ChgDeviceGuard guard(out);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "out is not a CUDA device pointer");
+    return dtype == NDCHG_F64 ? launch_refined_lee<double>(pol, values, shape, strides, window, looks, out, stream)
+                              : launch_refined_lee<float>(pol, values, shape, strides, window, looks, out, stream);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }
