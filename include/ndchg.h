@@ -144,6 +144,36 @@ int ndchg_enl(const void* values, const int64_t shape[3], const int64_t strides[
 int ndchg_refined_lee(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
                       uint32_t window, double looks, void* out, void* stream);
 
+/* H / A / alpha eigen-decomposition (Cloude & Pottier, IEEE TGRS 35(1), 1997; dual-pol: Cloude, IEEE GRSL 4(2),
+ * 2007) of every sample (pixel, step) on its own.  `values` as above, in the band order of `pol`, which is
+ * NDCHG_POL_DUAL, NDCHG_POL_QUAD or their diagonal layouts (off-diagonal bands zero); NDCHG_POL_SINGLE is rejected
+ * (a 1 x 1 matrix has no decomposition).  `out` is a DEVICE array (rows, cols, k, n) of the data type, C-contiguous,
+ * written completely, not overlapping `values`: per sample, quad layouts n = 6: [H, A, alpha, l1, l2, l3]; dual
+ * layouts n = 4: [H, alpha, l1, l2].  Requires k >= 1.  Checks: pol, single-pol, shape and k, dtype, overlap, then
+ * the device pointer.
+ *
+ * Matrix: quad layouts read the lexicographic C3 of k = [S_hh, sqrt2 S_hv, S_vv] and decompose the Pauli coherency
+ * matrix T = A C A^H, A = [[1, 0, 1], [1, 0, -1], [0, sqrt2, 0]] / sqrt2:
+ *     T11 = (C11 + 2 Re C13 + C33) / 2,  T22 = (C11 - 2 Re C13 + C33) / 2,  T33 = C22,
+ *     T12 = (C11 - C33) / 2 - i Im C13,  T13 = (C12 + conj C23) / sqrt2,  T23 = (C12 - conj C23) / sqrt2.
+ * Dual layouts decompose the 2 x 2 covariance C2 itself (the first component is the first channel).  With tau = 1e-9:
+ *   1. l1 >= l2 (>= l3): the eigenvalues, each clamped to max(l, 0); s = sum of them.
+ *   2. A sample with a non-finite band gives NaN everywhere.  s = 0 gives NaN H, A, alpha and the (zero) eigenvalues.
+ *   3. H = -sum p_i log_b p_i, p_i = l_i / s, 0 log 0 = 0, b = 3 (quad) or 2 (dual): 0 <= H <= 1.
+ *   4. A = (l2 - l3) / (l2 + l3), or 0 when l2 <= tau s (quad only).
+ *   5. Consecutive eigenvalues with l_i - l_{i+1} <= tau s form one cluster (chained: all three can).
+ *   6. c_i = |e_i[0]|^2 of the unit eigenvector, except that every member of a cluster of m gets the (0, 0) entry of
+ *      the cluster's projector / m (so alpha does not depend on the basis of a repeated eigenvalue);
+ *      alpha_i = arccos(sqrt c_i) in degrees (sqrt c_i clamped to [0, 1]), alpha = sum p_i alpha_i.
+ * Arithmetic: inputs are read in the data type, everything else is double, each output is rounded once.  The bands
+ * are scaled by a power of two first (exact; the eigenvalues are scaled back), so no scale overflows.  Quad: cyclic
+ * complex Jacobi rotations until the off-diagonal Frobenius norm is <= 2^-52 ||T||_F (at most 16 sweeps).  Dual: the
+ * closed form l1 = (C11 + C22) / 2 + r, r = hypot((C11 - C22) / 2, |C12|), l2 = det / l1, and |e_1[0]|^2 =
+ * (l1 - C22) / (2 r), |e_2[0]|^2 = (l1 - C11) / (2 r), each formed without cancellation.  Not bit-identical to a
+ * LAPACK restatement; eigenvalues agree to ~1e-12 s where every eigenvalue gap is <= tau s or >= 1e-4 s. */
+int ndchg_h_a_alpha(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol, void* out,
+                    void* stream);
+
 const char* ndchg_last_error(void);
 
 #ifdef __cplusplus

@@ -34,7 +34,7 @@ FLT_SYMBOLS = ["ndflt_correlate", "ndflt_correlate1d", "ndflt_launch_count", "nd
 # every symbol include/ndchg.h declares (omnibus change detection, SURVEY.md 8(f) row N4)
 CHG_SYMBOLS = ["ndchg_change_detection", "ndchg_omnibus_probability", "ndchg_change_detection_pol",
                "ndchg_omnibus_probability_pol", "ndchg_change_direction", "ndchg_enl", "ndchg_refined_lee",
-               "ndchg_last_error"]
+               "ndchg_h_a_alpha", "ndchg_last_error"]
 
 
 class Info(ctypes.Structure):
@@ -144,6 +144,8 @@ def lib():
     L.ndchg_enl.restype = ctypes.c_int
     L.ndchg_refined_lee.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, ctypes.c_double, vp, vp]
     L.ndchg_refined_lee.restype = ctypes.c_int
+    L.ndchg_h_a_alpha.argtypes = [vp, i64p, i64p, ctypes.c_int, ctypes.c_int, vp, vp]
+    L.ndchg_h_a_alpha.restype = ctypes.c_int
     L.ndchg_last_error.argtypes = []
     L.ndchg_last_error.restype = ctypes.c_char_p
     _lib = L

@@ -677,6 +677,170 @@ refined_lee_kernel(const T* __restrict__ values, const long long rows, const lon
     }
 }
 
+// ---- H / A / alpha decomposition (ndchg_h_a_alpha, include/ndchg.h) ----------------------------------------------
+// One thread per sample (pixel, step), with 64-bit sample and element indices.  The bands are first scaled by a
+// power of two (exact) so that their largest magnitude lies in [1, 2): squares and determinants can then neither
+// overflow nor underflow, and the eigenvalues are scaled back exactly.  Quad layouts diagonalise the Pauli coherency
+// matrix T by cyclic complex Jacobi; alpha needs only |e_i[0]|^2, the first row of the accumulated rotation V
+// (T = V diag(lambda) V^H), so that row is all that is kept.  Dual layouts use the closed form of the 2 x 2 matrix.
+constexpr int HAA_THREADS = 256, HAA_MAX_SWEEPS = 16;
+constexpr double HAA_TAU = 1e-9;
+
+__host__ __device__ constexpr int haa_outputs(const int pol) {
+    return pol == NDCHG_POL_QUAD || pol == NDCHG_POL_QUAD_DIAGONAL ? 6 : 4;
+}
+
+// (x, y) <- (c x - s ph y, s x + c ph y): columns p and q of a row times the rotation of haa_rotate
+__device__ __forceinline__ void haa_rot(double2& x, double2& y, const double c, const double s, const double2 ph) {
+    const double2 py = make_double2(ph.x * y.x - ph.y * y.y, ph.x * y.y + ph.y * y.x);
+    const double2 nx = make_double2(c * x.x - s * py.x, c * x.y - s * py.y);
+    y = make_double2(s * x.x + c * py.x, s * x.y + c * py.y);
+    x = nx;
+}
+
+__device__ __forceinline__ double2 haa_conj(const double2 a) { return make_double2(a.x, -a.y); }
+
+// One Jacobi rotation J of the plane (P, Q), P < Q, that zeroes T[P][Q] = m e^(i phi): J = diag(1, e^(-i phi)) R
+// on (P, Q) with the real rotation R = [[c, s], [-s, c]] of Numerical Recipes' jacobi, T <- J^H T J, V <- V J.
+// d: the real diagonal; u[r]: the upper entry of the plane without index r (u[2] = T01, u[1] = T02, u[0] = T12);
+// v: row 0 of V.
+template <int P, int Q>
+__device__ __forceinline__ void haa_rotate(double d[3], double2 u[3], double2 v[3]) {
+    constexpr int R = 3 - P - Q;
+    const double m = hypot(u[R].x, u[R].y);
+    if (m == 0.0) return;
+    const double2 ph = make_double2(u[R].x / m, -u[R].y / m);
+    const double theta = (d[Q] - d[P]) / (2.0 * m);
+    const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + hypot(theta, 1.0));
+    const double c = 1.0 / hypot(t, 1.0), s = t * c;
+    d[P] -= t * m;
+    d[Q] += t * m;
+    u[R] = make_double2(0.0, 0.0);
+    // row R of T holds T[R][P] and T[R][Q]; below the diagonal they are the conjugates of the stored upper entries
+    double2 rp = R > P ? haa_conj(u[Q]) : u[Q], rq = R > Q ? haa_conj(u[P]) : u[P];
+    haa_rot(rp, rq, c, s, ph);
+    u[Q] = R > P ? haa_conj(rp) : rp;
+    u[P] = R > Q ? haa_conj(rq) : rq;
+    haa_rot(v[P], v[Q], c, s, ph);
+}
+
+template <typename T, int POL>
+__global__ void __launch_bounds__(HAA_THREADS)
+h_a_alpha_kernel(const T* __restrict__ values, const long long cols, const long long k, const long long samples,
+                 const long long s0, const long long s1, const long long s2, const long long s3, T* __restrict__ out) {
+    constexpr int B = pol_bands(POL), NO = haa_outputs(POL);
+    constexpr bool QUAD = POL == NDCHG_POL_QUAD || POL == NDCHG_POL_QUAD_DIAGONAL;
+    constexpr int K = QUAD ? 3 : 2;                                      // matrix size
+    const long long g = (long long)blockIdx.x * HAA_THREADS + threadIdx.x;
+    if (g >= samples) return;
+    const long long pix = g / k, t = g - pix * k, i = pix / cols, j = pix - i * cols;
+    const T* src = values + i * s0 + j * s1 + t * s2;
+    T* o = out + g * NO;
+    double x[B], amax = 0.0;
+    bool finite = true;
+#pragma unroll
+    for (int b = 0; b < B; ++b) {
+        x[b] = double(src[b * s3]);
+        finite = finite && isfinite(x[b]);
+        amax = fmax(amax, fabs(x[b]));
+    }
+    if (!finite) {
+#pragma unroll
+        for (int q = 0; q < NO; ++q) o[q] = T(CUDART_NAN);
+        return;
+    }
+    const int e = amax > 0.0 ? ilogb(amax) : 0;
+#pragma unroll
+    for (int b = 0; b < B; ++b) x[b] = scalbn(x[b], -e);
+    double lam[K], w[K];                                                 // eigenvalues (descending), |e_i[0]|^2
+    bool tie[K - 1];
+    if constexpr (QUAD) {
+        // C3 = [C11, C12, C13, C22, C23, C33]; the diagonal layout has no off-diagonal bands
+        const double c11 = x[0], c22 = x[POL == NDCHG_POL_QUAD ? 5 : 1], c33 = x[POL == NDCHG_POL_QUAD ? 8 : 2];
+        const double c12r = POL == NDCHG_POL_QUAD ? x[1] : 0.0, c12i = POL == NDCHG_POL_QUAD ? x[2] : 0.0;
+        const double c13r = POL == NDCHG_POL_QUAD ? x[3] : 0.0, c13i = POL == NDCHG_POL_QUAD ? x[4] : 0.0;
+        const double c23r = POL == NDCHG_POL_QUAD ? x[6] : 0.0, c23i = POL == NDCHG_POL_QUAD ? x[7] : 0.0;
+        const double r2 = 0.70710678118654752440;                        // 1 / sqrt(2)
+        double d[3] = {0.5 * (c11 + 2.0 * c13r + c33), 0.5 * (c11 - 2.0 * c13r + c33), c22};
+        double2 u[3] = {make_double2((c12r - c23r) * r2, (c12i + c23i) * r2),          // T23 = (C12 - conj C23) / sqrt 2
+                        make_double2((c12r + c23r) * r2, (c12i - c23i) * r2),          // T13 = (C12 + conj C23) / sqrt 2
+                        make_double2(0.5 * (c11 - c33), -c13i)};                         // T12 = (C11 - C33) / 2 - i Im C13
+        double2 v[3] = {make_double2(1.0, 0.0), make_double2(0.0, 0.0), make_double2(0.0, 0.0)};
+        // until the off-diagonal Frobenius norm is <= eps ||T||_F
+        constexpr double eps2 = 2.220446049250313e-16 * 2.220446049250313e-16;
+        for (int sweep = 0; sweep < HAA_MAX_SWEEPS; ++sweep) {
+            const double off = 2.0 * (u[0].x * u[0].x + u[0].y * u[0].y + u[1].x * u[1].x + u[1].y * u[1].y +
+                                      u[2].x * u[2].x + u[2].y * u[2].y);
+            if (off <= eps2 * (d[0] * d[0] + d[1] * d[1] + d[2] * d[2] + off)) break;
+            haa_rotate<0, 1>(d, u, v);
+            haa_rotate<0, 2>(d, u, v);
+            haa_rotate<1, 2>(d, u, v);
+        }
+#pragma unroll
+        for (int q = 0; q < 3; ++q) {
+            lam[q] = d[q];
+            w[q] = v[q].x * v[q].x + v[q].y * v[q].y;
+        }
+        // sort descending, |e[0]|^2 along
+#define HAA_ORDER(a, b)                                                                 \
+        if (lam[a] < lam[b]) {                                                          \
+            const double tl = lam[a], tw = w[a];                                        \
+            lam[a] = lam[b]; w[a] = w[b]; lam[b] = tl; w[b] = tw;                       \
+        }
+        HAA_ORDER(0, 1) HAA_ORDER(1, 2) HAA_ORDER(0, 1)
+#undef HAA_ORDER
+    } else {
+        // C2 = [[C11, C12], [conj C12, C22]]: lambda = (C11 + C22) / 2 +- r, r = hypot((C11 - C22) / 2, |C12|);
+        // lambda2 = det / lambda1 (no cancellation); |e_1[0]|^2 = (lambda1 - C22) / (2 r), |e_2[0]|^2 =
+        // (lambda1 - C11) / (2 r), each side formed without cancellation, (lambda1 - C11)(lambda1 - C22) = |C12|^2
+        const double c11 = x[0], c22 = x[POL == NDCHG_POL_DUAL ? 3 : 1];
+        const double b2 = POL == NDCHG_POL_DUAL ? x[1] * x[1] + x[2] * x[2] : 0.0;
+        const double delta = 0.5 * (c11 - c22), r = hypot(delta, sqrt(b2));
+        lam[0] = 0.5 * (c11 + c22) + r;
+        lam[1] = lam[0] > 0.0 ? (c11 * c22 - b2) / lam[0] : lam[0];      // lambda1 <= 0: s = 0 below
+        const double a1 = delta >= 0.0 ? delta + r : b2 / (r - delta);   // lambda1 - C22
+        const double a2 = delta >= 0.0 ? b2 / (delta + r) : r - delta;   // lambda1 - C11
+        w[0] = a1 / (2.0 * r);
+        w[1] = a2 / (2.0 * r);
+    }
+    double s = 0.0;
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        lam[q] = fmax(lam[q], 0.0);
+        s += lam[q];
+    }
+#pragma unroll
+    for (int q = 0; q < K - 1; ++q) tie[q] = lam[q] - lam[q + 1] <= HAA_TAU * s;
+    double H = CUDART_NAN, A = CUDART_NAN, alpha = CUDART_NAN;
+    if (s > 0.0) {
+        // the tie clusters share the mean of their |e[0]|^2: the (0, 0) entry of the cluster's projector / m
+        if constexpr (K == 2) {
+            if (tie[0]) w[0] = w[1] = 0.5;
+        } else {
+            if (tie[0] && tie[1]) w[0] = w[1] = w[2] = (w[0] + w[1] + w[2]) / 3.0;
+            else if (tie[0]) w[0] = w[1] = 0.5 * (w[0] + w[1]);
+            else if (tie[1]) w[1] = w[2] = 0.5 * (w[1] + w[2]);
+        }
+        H = 0.0;
+        alpha = 0.0;
+#pragma unroll
+        for (int q = 0; q < K; ++q) {
+            const double p = lam[q] / s;
+            if (p > 0.0) H -= p * log(p);
+            alpha += p * acos(fmin(fmax(sqrt(w[q]), 0.0), 1.0));
+        }
+        H /= K == 3 ? 1.0986122886681098 : 0.69314718055994531;         // ln 3, ln 2
+        alpha *= 57.295779513082321;                                     // 180 / pi
+        if constexpr (K == 3) A = lam[1] <= HAA_TAU * s ? 0.0 : (lam[1] - lam[2]) / (lam[1] + lam[2]);
+    }
+    int q = 0;
+    o[q++] = T(H);
+    if constexpr (K == 3) o[q++] = T(A);
+    o[q++] = T(alpha);
+#pragma unroll
+    for (int r = 0; r < K; ++r) o[q++] = T(scalbn(lam[r], e));
+}
+
 }  // namespace ndchg
 
 struct ChgDeviceGuard {
@@ -914,8 +1078,10 @@ static int launch_refined_lee(int pol, const void* values, const int64_t* shape,
     }
 }
 
-// true if the bytes `values` spans (any strides, including negative ones) meet the C-contiguous output
-static bool lee_overlap(const void* values, const int64_t* shape, const int64_t* strides, int bands, size_t elem, const void* out) {
+// true if the bytes `values` spans (any strides, including negative ones) meet the C-contiguous output of `outs`
+// values per sample
+static bool lee_overlap(const void* values, const int64_t* shape, const int64_t* strides, int bands, size_t elem, const void* out,
+                        int outs) {
     const int64_t n[4] = {shape[0], shape[1], shape[2], bands};
     const char* lo = (const char*)values;
     const char* hi = lo + elem;
@@ -925,7 +1091,7 @@ static bool lee_overlap(const void* values, const int64_t* shape, const int64_t*
         else hi += ext;
     }
     const char* olo = (const char*)out;
-    const char* ohi = olo + shape[0] * shape[1] * shape[2] * bands * int64_t(elem);
+    const char* ohi = olo + shape[0] * shape[1] * shape[2] * outs * int64_t(elem);
     return lo < ohi && olo < hi;
 }
 
@@ -943,12 +1109,56 @@ extern "C" int ndchg_refined_lee(const void* values, const int64_t shape[3], con
     if (!(looks > 0.0) || !std::isfinite(looks))
         return chg_fail(NDNLM_EINVAL, "the number of looks must be finite and > 0, got %g", looks);
     if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
-    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out))
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::pol_bands(pol)))
         return chg_fail(NDNLM_EINVAL, "out must not overlap values");
     ChgDeviceGuard guard(out);
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "out is not a CUDA device pointer");
     return dtype == NDCHG_F64 ? launch_refined_lee<double>(pol, values, shape, strides, window, looks, out, stream)
                               : launch_refined_lee<float>(pol, values, shape, strides, window, looks, out, stream);
+}
+
+template <typename T, int POL>
+static int launch_h_a_alpha(const void* values, const int64_t* shape, const int64_t* strides, void* out, void* stream) {
+    const long long samples = shape[0] * shape[1] * shape[2];
+    const long long blocks = (samples + ndchg::HAA_THREADS - 1) / ndchg::HAA_THREADS;
+    if (blocks > 0x7fffffffLL) return chg_fail(NDNLM_EINVAL, "%lld samples are too many for ndchg_h_a_alpha", samples);
+    ndchg::h_a_alpha_kernel<T, POL><<<unsigned(blocks), ndchg::HAA_THREADS, 0, (cudaStream_t)stream>>>(
+        (const T*)values, shape[1], shape[2], samples, strides[0], strides[1], strides[2], strides[3], (T*)out);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return NDNLM_OK;
+}
+
+template <typename T>
+static int launch_h_a_alpha(int pol, const void* values, const int64_t* shape, const int64_t* strides, void* out, void* stream) {
+    switch (pol) {
+        case NDCHG_POL_DUAL: return launch_h_a_alpha<T, NDCHG_POL_DUAL>(values, shape, strides, out, stream);
+        case NDCHG_POL_QUAD: return launch_h_a_alpha<T, NDCHG_POL_QUAD>(values, shape, strides, out, stream);
+        case NDCHG_POL_DUAL_DIAGONAL: return launch_h_a_alpha<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, out, stream);
+        case NDCHG_POL_QUAD_DIAGONAL: return launch_h_a_alpha<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, out, stream);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+extern "C" int ndchg_h_a_alpha(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                               void* out, void* stream) {
+    if (!values || !shape || !strides || !out) return chg_fail(NDNLM_EINVAL, "null argument");
+    if (pol < NDCHG_POL_DUAL || pol > NDCHG_POL_QUAD_DIAGONAL) return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    if (pol == NDCHG_POL_SINGLE)
+        return chg_fail(NDNLM_EINVAL, "single-pol data have no H / A / alpha decomposition (a 1 x 1 matrix has no eigenvectors)");
+    // every extent below 2^40: the element count (x 9 bands) stays far inside int64
+    if (shape[0] < 1 || shape[1] < 1 || shape[0] >= (1LL << 40) || shape[1] >= (1LL << 40) ||
+        double(shape[0]) * double(shape[1]) >= double(1LL << 40))
+        return chg_fail(NDNLM_EINVAL, "shape out of range");
+    if (shape[2] < 1 || double(shape[0]) * double(shape[1]) * double(shape[2]) >= double(1LL << 56))
+        return chg_fail(NDNLM_EINVAL, "the H / A / alpha decomposition needs at least 1 time step (and fewer than 2^56 samples)");
+    if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::haa_outputs(pol)))
+        return chg_fail(NDNLM_EINVAL, "out must not overlap values");
+    ChgDeviceGuard guard(out);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "out is not a CUDA device pointer");
+    return dtype == NDCHG_F64 ? launch_h_a_alpha<double>(pol, values, shape, strides, out, stream)
+                              : launch_h_a_alpha<float>(pol, values, shape, strides, out, stream);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }
