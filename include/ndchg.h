@@ -174,6 +174,56 @@ int ndchg_refined_lee(const void* values, const int64_t shape[3], const int64_t 
 int ndchg_h_a_alpha(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol, void* out,
                     void* stream);
 
+/* Cloude-Pottier zone of every sample in the H / alpha plane (Lee, Grunes, Ainsworth, Du, Schuler & Cloude, IEEE
+ * TGRS 37(5), 1999), the initial classes of ndchg_wishart_classify.  `values` and `pol` as for ndchg_h_a_alpha
+ * (NDCHG_POL_SINGLE is rejected); `zones` is a DEVICE uint8 array (rows, cols, k), C-contiguous, written completely,
+ * not overlapping `values`.  The zone is a pure function of the H, A and alpha that ndchg_h_a_alpha returns for the
+ * sample in the data type, compared with the thresholds in double (Lee et al.'s numbering):
+ *     H >= 0.9:        1: alpha >= 55          2: 40 <= alpha < 55     3: alpha < 40 (not feasible, normally empty)
+ *     0.5 <= H < 0.9:  4: alpha >= 50          5: 40 <= alpha < 50     6: alpha < 40
+ *     H < 0.5:         7: alpha >= 47.5        8: 42.5 <= alpha < 47.5 9: alpha < 42.5
+ * A sample with NaN H or alpha gets zone 0.  `anisotropy` = 1 (quad layouts only; 0 or 1) adds 9 where A > 0.5:
+ * labels 1..18, the 16 classes of the H / A / alpha Wishart initialisation plus the two normally empty zones.  Which
+ * side of each boundary a value on it belongs to is this project's convention (no bit-parity with any other tool
+ * is claimed).  The dual layouts use the same plane on Cloude's dual-pol H / alpha; that is a convention too, since
+ * the feasible region of the dual-pol plane differs.  Checks: pol, single-pol, anisotropy, shape and k, dtype,
+ * overlap, then the device pointer.  ndchg_h_a_alpha runs into device scratch of at most 2^24 samples at a time. */
+int ndchg_h_alpha_zones(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                        int anisotropy, uint8_t* zones, void* stream);
+
+/* Unsupervised Wishart classification (Lee et al., IEEE TGRS 37(5), 1999): k-means with the complex Wishart distance
+ * from the initial labels `labels`, one set of K = `classes` centres for every sample (pixel, step) of the series,
+ * so a label means the same on every date.  `values` as for ndchg_h_a_alpha (dual, quad and the diagonal layouts;
+ * NDCHG_POL_SINGLE is rejected); p = 2 (dual layouts) or 3 (quad layouts); B bands.  `labels` is a DEVICE uint8
+ * array (rows, cols, k), C-contiguous, not overlapping `values`: read (0 = unlabelled, 1..K), then overwritten with
+ * the result.  `centres` (K x B doubles, row-major), `counts` (K int64) and `iterations` (one uint32) are DEVICE
+ * buffers; they describe the labels returned.  Limits: 1 <= classes <= 32, tol in [0, 1].
+ *   Valid samples: every band finite and the trace (the diagonal bands added left to right) > 0.  Invalid samples
+ *     always get label 0, and no sum counts them.
+ *   Iteration 0: V_m = the band-wise mean of the valid samples labelled m (m = 1..K).  A label > K anywhere is
+ *     NDNLM_EINVAL and nothing is written.
+ *   Active class: count_m >= 1 and det V_m > 1e-12 (tr V_m / p)^p, with det the Hermitian determinant of
+ *     ndchg_change_direction's m2 / m3 (the product of the diagonal for the diagonal layouts) and (tr / p)^p formed
+ *     as q q (q) from q = tr / p.  No active class after iteration 0 is NDNLM_EINVAL.
+ *   Distance (the covariance domain; it equals the distance on the Pauli T, since T = A C A^H with A unitary):
+ *     d_m(C) = ln det V_m + tr(V_m^-1 C) = g_m + sum_b w_mb x_b, with g_m = ln det V_m, W = V_m^-1 = adj(V_m) / det
+ *     V_m, and w_mb = W_ii for the band C_ii, 2 Re W_ij for Re C_ij and 2 Im W_ij for Im C_ij.  Evaluated as
+ *     acc = g_m, then acc = acc + w_mb x_b in band order, each a separately rounded double operation (no FMA).
+ *   Iterations 1..max_iter: every valid sample takes the argmin of d_m over the active classes (a tie goes to the
+ *     lowest m); the samples whose label changed (0 -> m included) are counted; the centres are recomputed from the
+ *     new labels.  The loop stops after iteration i when changed <= tol * (number of valid samples), or when no class
+ *     is active any more; `iterations` = the last i run (0 when max_iter = 0).
+ *   Centres: K x B means in double, NaN for inactive classes; counts: the valid samples of each label.
+ * Rounding: inputs are read in the data type, everything else is double; the sums of every pass are formed in a fixed
+ * order (fixed chunks of samples, a fixed order inside a chunk, a fixed tree over the chunks), so a call is bit-identical
+ * from run to run and for any strides of the same data.  ln is CUDA's `log`, which is not correctly rounded.
+ * Checks: pol, single-pol, shape and k, dtype, classes, tol, overlap, then the device pointers.  The call waits for
+ * iteration 0 on `stream` (to report a label > K or no active class) and enqueues the iterations asynchronously: a
+ * device flag, set when the loop stops, turns the later launches into early returns. */
+int ndchg_wishart_classify(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                           uint8_t* labels, uint32_t classes, uint32_t max_iter, double tol, double* centres,
+                           int64_t* counts, uint32_t* iterations, void* stream);
+
 const char* ndchg_last_error(void);
 
 #ifdef __cplusplus

@@ -841,6 +841,269 @@ h_a_alpha_kernel(const T* __restrict__ values, const long long cols, const long 
     for (int r = 0; r < K; ++r) o[q++] = T(scalbn(lam[r], e));
 }
 
+// ---- H / alpha zones and the Wishart classification (ndchg_h_alpha_zones, ndchg_wishart_classify) -----------------
+// Zones: h_a_alpha_kernel runs unchanged into device scratch (ZONE_CHUNK samples at a time), then one thread per
+// sample reads its H, A, alpha.  Wishart: three kernels per iteration on one stream.  `wishart_assign_kernel` reads
+// the cube once: one CTA owns a fixed chunk of WIS_CHUNK consecutive samples (the partition depends on the sample
+// count only, never on the device), each warp 32 samples at a time.  A lane takes the argmin of its sample, then the
+// warp stages its 32 (label, bands) in shared memory and lane e of lane group q adds accumulator column e (a band,
+// or the count) of samples q, q + Q, ... in lane order into the group's own K x (B + 1) copy.  The copies are added
+// in (warp, group) order into one partial per chunk; `wishart_reduce_kernel` adds the chunk partials of every
+// accumulator in a fixed tree, and `wishart_centres_kernel` (one warp) turns the sums into the next (g, w) table.
+// No floating-point atomics, so the sums are bit-identical from run to run, on any B200 and for any strides.
+constexpr int WIS_THREADS = 256, WIS_WARPS = WIS_THREADS / 32, WIS_GROUPS = 16, WIS_MAX_CLASSES = 32;
+constexpr long long WIS_CHUNK = (long long)WIS_THREADS * WIS_GROUPS;    // samples per CTA, i.e. per chunk of the sums
+constexpr long long ZONE_CHUNK = 1LL << 24;
+constexpr int WIS_REDUCE_THREADS = 256;
+
+// lane groups of a warp in the accumulation: Q groups of B + 1 lanes
+__host__ __device__ constexpr int wis_groups(const int pol) { return 32 / (pol_bands(pol) + 1); }
+
+__host__ __device__ constexpr size_t wis_smem(const int pol, const int K) {
+    return sizeof(double) * size_t(WIS_WARPS) * wis_groups(pol) * K * (pol_bands(pol) + 1);
+}
+
+// device state of one ndchg_wishart_classify call; the sums and the chunk partials follow it in the same scratch
+struct WisState {
+    unsigned long long changed;                      // samples whose label changed in the current pass
+    unsigned long long valid;                        // valid samples (counted in iteration 0)
+    unsigned done;                                   // the loop has stopped: every later launch returns at once
+    unsigned bad;                                    // an initial label > K
+    unsigned active;                                 // active classes after the last centres kernel
+    int act[WIS_MAX_CLASSES];
+    double g[WIS_MAX_CLASSES];                       // ln det V_m
+    double w[WIS_MAX_CLASSES * 9];                   // [K][B]: the weights of the distance
+};
+
+template <typename T, int POL>
+__global__ void __launch_bounds__(HAA_THREADS)
+h_alpha_zone_kernel(const T* __restrict__ haa, const long long n, const int anisotropy, unsigned char* __restrict__ zones) {
+    constexpr bool QUAD = POL == NDCHG_POL_QUAD || POL == NDCHG_POL_QUAD_DIAGONAL;
+    const long long g = (long long)blockIdx.x * HAA_THREADS + threadIdx.x;
+    if (g >= n) return;
+    const T* o = haa + g * haa_outputs(POL);
+    const double H = double(o[0]), alpha = double(o[QUAD ? 2 : 1]);
+    unsigned char z = 0;
+    if (!isnan(H) && !isnan(alpha)) {
+        if (H >= 0.9) z = alpha >= 55.0 ? 1 : alpha >= 40.0 ? 2 : 3;
+        else if (H >= 0.5) z = alpha >= 50.0 ? 4 : alpha >= 40.0 ? 5 : 6;
+        else z = alpha >= 47.5 ? 7 : alpha >= 42.5 ? 8 : 9;
+        if (QUAD && anisotropy && double(o[1]) > 0.5) z += 9;
+    }
+    zones[g] = z;
+}
+
+// sets `bad` (and `done`) if any initial label exceeds K
+__global__ void __launch_bounds__(256)
+wishart_check_kernel(const unsigned char* __restrict__ labels, const long long n, const int K, WisState* st) {
+    bool bad = false;
+    for (long long g = (long long)blockIdx.x * 256 + threadIdx.x; g < n; g += (long long)gridDim.x * 256) bad |= labels[g] > K;
+    if (__syncthreads_or(bad) && threadIdx.x == 0) {
+        st->bad = 1;
+        st->done = 1;
+    }
+}
+
+// One pass over the cube.  ASSIGN = false is iteration 0: the initial labels are kept (invalid samples set to 0) and
+// the valid samples are counted; ASSIGN = true takes the argmin and counts the changed labels.  Either way the pass
+// accumulates, per label, the band sums and the count of its valid samples into partials[a * nchunk + chunk].
+// FLAT: the (rows, cols, k) axes collapse into one of stride s2, so sample g starts at element g * s2.
+template <typename T, int POL, bool ASSIGN>
+__global__ void __launch_bounds__(WIS_THREADS)
+wishart_assign_kernel(const T* __restrict__ values, const long long cols, const long long k, const long long samples,
+                      const long long s0, const long long s1, const long long s2, const long long s3, const bool flat,
+                      unsigned char* __restrict__ labels, WisState* __restrict__ st, const int K,
+                      double* __restrict__ partials, const long long nchunk) {
+    constexpr int B = pol_bands(POL), E = B + 1, Q = wis_groups(POL);
+    __shared__ double tab_g[WIS_MAX_CLASSES], tab_w[WIS_MAX_CLASSES * B];
+    __shared__ int tab_act[WIS_MAX_CLASSES];
+    __shared__ T stage[WIS_WARPS][32][B];
+    __shared__ unsigned char slab[WIS_WARPS][32];
+    __shared__ unsigned long long cta_count;
+    extern __shared__ double acc[];                                      // [WIS_WARPS][Q][K][E]
+    if (st->done) return;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (ASSIGN) {
+        for (int q = tid; q < K * B; q += WIS_THREADS) tab_w[q] = st->w[q];
+        if (tid < K) {
+            tab_g[tid] = st->g[tid];
+            tab_act[tid] = st->act[tid];
+        }
+    }
+    for (int q = tid; q < WIS_WARPS * Q * K * E; q += WIS_THREADS) acc[q] = 0.0;
+    if (tid == 0) cta_count = 0;
+    __syncthreads();
+    double* myacc = acc + warp * Q * K * E;
+    const int grp = lane / E, col = lane - grp * E;                       // the lane's copy and accumulator column
+    unsigned count = 0;
+    const long long base = (long long)blockIdx.x * WIS_CHUNK + warp * (32 * WIS_GROUPS);
+    for (int r = 0; r < WIS_GROUPS; ++r) {
+        const long long g = base + r * 32 + lane;
+        int lab = 0;
+        if (g < samples) {
+            long long off;
+            if (flat) {
+                off = g * s2;
+            } else {
+                const long long pix = g / k, t = g - pix * k, i = pix / cols, j = pix - i * cols;
+                off = i * s0 + j * s1 + t * s2;
+            }
+            const T* src = values + off;
+            double x[B];
+            bool finite = true;
+#pragma unroll
+            for (int b = 0; b < B; ++b) {
+                const T v = src[b * s3];
+                stage[warp][lane][b] = v;
+                x[b] = double(v);
+                finite = finite && isfinite(x[b]);
+            }
+            double tr = x[lee_diagonal_band(POL, 0)];
+#pragma unroll
+            for (int d = 1; d < lee_diagonals(POL); ++d) tr = add_(tr, x[lee_diagonal_band(POL, d)]);
+            const int old = labels[g];
+            if (finite && tr > 0.0) {
+                if (ASSIGN) {
+                    double best = CUDART_INF;
+                    for (int m = 0; m < K; ++m) {
+                        if (!tab_act[m]) continue;
+                        const double* w = tab_w + m * B;
+                        double d = tab_g[m];
+#pragma unroll
+                        for (int b = 0; b < B; ++b) d = add_(d, mul_(w[b], x[b]));
+                        if (d < best) {
+                            best = d;
+                            lab = m + 1;
+                        }
+                    }
+                    if (lab != old) {
+                        labels[g] = (unsigned char)lab;
+                        ++count;
+                    }
+                } else {
+                    lab = old;
+                    ++count;
+                }
+            } else if (!ASSIGN && old != 0) {
+                labels[g] = 0;
+            }
+        }
+        slab[warp][lane] = (unsigned char)lab;
+        __syncwarp();
+        if (grp < Q) {
+            double* a = myacc + grp * K * E + col;
+            for (int s = grp; s < 32; s += Q) {
+                const int m = slab[warp][s];
+                if (m) a[(m - 1) * E] = add_(a[(m - 1) * E], col < B ? double(stage[warp][s][col < B ? col : 0]) : 1.0);
+            }
+        }
+        __syncwarp();
+    }
+    count = __reduce_add_sync(0xffffffffu, count);
+    if (lane == 0 && count) atomicAdd(&cta_count, (unsigned long long)count);
+    __syncthreads();
+    if (tid == 0 && cta_count) atomicAdd(ASSIGN ? &st->changed : &st->valid, cta_count);
+    for (int a = tid; a < K * E; a += WIS_THREADS) {
+        double s = 0.0;
+        for (int c = 0; c < WIS_WARPS * Q; ++c) s = add_(s, acc[c * K * E + a]);
+        partials[a * nchunk + blockIdx.x] = s;
+    }
+}
+
+// sums[a] = the chunk partials of accumulator a = blockIdx.x, added in a fixed tree
+__global__ void __launch_bounds__(WIS_REDUCE_THREADS)
+wishart_reduce_kernel(const double* __restrict__ partials, const long long nchunk, double* __restrict__ sums,
+                      const WisState* __restrict__ st) {
+    __shared__ double red[WIS_REDUCE_THREADS];
+    if (st->done) return;
+    const int tid = threadIdx.x;
+    const double* p = partials + blockIdx.x * nchunk;
+    double s = 0.0;
+    for (long long c = tid; c < nchunk; c += WIS_REDUCE_THREADS) s = add_(s, p[c]);
+    red[tid] = s;
+    __syncthreads();
+    for (int h = WIS_REDUCE_THREADS / 2; h > 0; h >>= 1) {
+        if (tid < h) red[tid] = add_(red[tid], red[tid + h]);
+        __syncthreads();
+    }
+    if (tid == 0) sums[blockIdx.x] = red[0];
+}
+
+// One warp, thread m = class m + 1: the mean V, det V, the active flag, W = adj(V) / det V and the (g, w) table of
+// the next pass; writes the outputs and decides whether the loop stops after iteration `it`.
+template <int POL>
+__global__ void __launch_bounds__(32)
+wishart_centres_kernel(WisState* __restrict__ st, const double* __restrict__ sums, const int K, const unsigned it,
+                       const unsigned max_iter, const double tol, double* __restrict__ centres,
+                       long long* __restrict__ counts, unsigned* __restrict__ iterations) {
+    constexpr int B = pol_bands(POL), E = B + 1, P = lee_diagonals(POL);
+    if (st->done) return;
+    const int m = threadIdx.x;
+    bool act = false;
+    if (m < K) {
+        const double n = sums[m * E + B];
+        double V[B];
+#pragma unroll
+        for (int b = 0; b < B; ++b) V[b] = __ddiv_rn(sums[m * E + b], n);
+        double tr = V[lee_diagonal_band(POL, 0)];
+#pragma unroll
+        for (int d = 1; d < P; ++d) tr = add_(tr, V[lee_diagonal_band(POL, d)]);
+        const double q = __ddiv_rn(tr, double(P));
+        const double qp = P == 2 ? mul_(q, q) : mul_(mul_(q, q), q);
+        double det, w[B];
+        if constexpr (POL == NDCHG_POL_DUAL) {
+            const double a = V[0], br = V[1], bi = V[2], d = V[3];
+            det = sub_(mul_(a, d), add_(mul_(br, br), mul_(bi, bi)));
+            w[0] = __ddiv_rn(d, det);
+            w[1] = mul_(-2.0, __ddiv_rn(br, det));
+            w[2] = mul_(-2.0, __ddiv_rn(bi, det));
+            w[3] = __ddiv_rn(a, det);
+        } else if constexpr (POL == NDCHG_POL_QUAD) {
+            const double a = V[0], br = V[1], bi = V[2], cr = V[3], ci = V[4], d = V[5], er = V[6], ei = V[7], g = V[8];
+            const double re_bec = add_(mul_(sub_(mul_(br, er), mul_(bi, ei)), cr), mul_(add_(mul_(br, ei), mul_(bi, er)), ci));
+            const double e2 = add_(mul_(er, er), mul_(ei, ei)), c2 = add_(mul_(cr, cr), mul_(ci, ci));
+            const double b2 = add_(mul_(br, br), mul_(bi, bi));
+            det = add_(mul_(mul_(a, d), g), mul_(2.0, re_bec));
+            det = sub_(det, mul_(a, e2));
+            det = sub_(det, mul_(d, c2));
+            det = sub_(det, mul_(g, b2));
+            // adj(V) / det: W12 = (c conj(e) - b g) / det, W13 = (b e - c d) / det, W23 = (c conj(b) - a e) / det
+            w[0] = __ddiv_rn(sub_(mul_(d, g), e2), det);
+            w[5] = __ddiv_rn(sub_(mul_(a, g), c2), det);
+            w[8] = __ddiv_rn(sub_(mul_(a, d), b2), det);
+            w[1] = mul_(2.0, __ddiv_rn(sub_(add_(mul_(cr, er), mul_(ci, ei)), mul_(br, g)), det));
+            w[2] = mul_(2.0, __ddiv_rn(sub_(sub_(mul_(ci, er), mul_(cr, ei)), mul_(bi, g)), det));
+            w[3] = mul_(2.0, __ddiv_rn(sub_(sub_(mul_(br, er), mul_(bi, ei)), mul_(cr, d)), det));
+            w[4] = mul_(2.0, __ddiv_rn(sub_(add_(mul_(br, ei), mul_(bi, er)), mul_(ci, d)), det));
+            w[6] = mul_(2.0, __ddiv_rn(sub_(add_(mul_(cr, br), mul_(ci, bi)), mul_(a, er)), det));
+            w[7] = mul_(2.0, __ddiv_rn(sub_(sub_(mul_(ci, br), mul_(cr, bi)), mul_(a, ei)), det));
+        } else {
+            det = V[0];
+#pragma unroll
+            for (int b = 1; b < B; ++b) det = mul_(det, V[b]);
+#pragma unroll
+            for (int b = 0; b < B; ++b) w[b] = __ddiv_rn(1.0, V[b]);
+        }
+        act = n >= 1.0 && det > mul_(1e-12, qp);
+#pragma unroll
+        for (int b = 0; b < B; ++b) {
+            centres[m * B + b] = act ? V[b] : CUDART_NAN;
+            st->w[m * B + b] = act ? w[b] : 0.0;
+        }
+        st->g[m] = act ? log(det) : 0.0;
+        st->act[m] = act;
+        counts[m] = (long long)n;
+    }
+    const unsigned nact = __popc(__ballot_sync(0xffffffffu, act));
+    if (m == 0) {
+        const unsigned long long changed = st->changed;
+        st->active = nact;
+        st->changed = 0;
+        *iterations = it;
+        if (it >= max_iter || nact == 0 || (it >= 1 && double(changed) <= __dmul_rn(tol, double(st->valid)))) st->done = 1;
+    }
+}
+
 }  // namespace ndchg
 
 struct ChgDeviceGuard {
@@ -1079,9 +1342,9 @@ static int launch_refined_lee(int pol, const void* values, const int64_t* shape,
 }
 
 // true if the bytes `values` spans (any strides, including negative ones) meet the C-contiguous output of `outs`
-// values per sample
+// values of `oelem` bytes per sample
 static bool lee_overlap(const void* values, const int64_t* shape, const int64_t* strides, int bands, size_t elem, const void* out,
-                        int outs) {
+                        int outs, size_t oelem) {
     const int64_t n[4] = {shape[0], shape[1], shape[2], bands};
     const char* lo = (const char*)values;
     const char* hi = lo + elem;
@@ -1091,7 +1354,7 @@ static bool lee_overlap(const void* values, const int64_t* shape, const int64_t*
         else hi += ext;
     }
     const char* olo = (const char*)out;
-    const char* ohi = olo + shape[0] * shape[1] * shape[2] * outs * int64_t(elem);
+    const char* ohi = olo + shape[0] * shape[1] * shape[2] * outs * int64_t(oelem);
     return lo < ohi && olo < hi;
 }
 
@@ -1109,7 +1372,8 @@ extern "C" int ndchg_refined_lee(const void* values, const int64_t shape[3], con
     if (!(looks > 0.0) || !std::isfinite(looks))
         return chg_fail(NDNLM_EINVAL, "the number of looks must be finite and > 0, got %g", looks);
     if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
-    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::pol_bands(pol)))
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::pol_bands(pol),
+                    dtype == NDCHG_F64 ? 8 : 4))
         return chg_fail(NDNLM_EINVAL, "out must not overlap values");
     ChgDeviceGuard guard(out);
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "out is not a CUDA device pointer");
@@ -1153,12 +1417,209 @@ extern "C" int ndchg_h_a_alpha(const void* values, const int64_t shape[3], const
     if (shape[2] < 1 || double(shape[0]) * double(shape[1]) * double(shape[2]) >= double(1LL << 56))
         return chg_fail(NDNLM_EINVAL, "the H / A / alpha decomposition needs at least 1 time step (and fewer than 2^56 samples)");
     if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
-    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::haa_outputs(pol)))
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, out, ndchg::haa_outputs(pol),
+                    dtype == NDCHG_F64 ? 8 : 4))
         return chg_fail(NDNLM_EINVAL, "out must not overlap values");
     ChgDeviceGuard guard(out);
     if (!guard.ok) return chg_fail(NDNLM_EINVAL, "out is not a CUDA device pointer");
     return dtype == NDCHG_F64 ? launch_h_a_alpha<double>(pol, values, shape, strides, out, stream)
                               : launch_h_a_alpha<float>(pol, values, shape, strides, out, stream);
+}
+
+// the checks ndchg_h_alpha_zones and ndchg_wishart_classify share with ndchg_h_a_alpha, in its order: pol, single-pol,
+// (the caller's own checks), shape and k, dtype
+static int check_decomposable(int pol) {
+    if (pol < NDCHG_POL_DUAL || pol > NDCHG_POL_QUAD_DIAGONAL) return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    if (pol == NDCHG_POL_SINGLE)
+        return chg_fail(NDNLM_EINVAL, "single-pol data have no H / A / alpha decomposition (a 1 x 1 matrix has no eigenvectors)");
+    return NDNLM_OK;
+}
+
+static int check_samples(const int64_t* shape, int dtype) {
+    if (shape[0] < 1 || shape[1] < 1 || shape[0] >= (1LL << 40) || shape[1] >= (1LL << 40) ||
+        double(shape[0]) * double(shape[1]) >= double(1LL << 40))
+        return chg_fail(NDNLM_EINVAL, "shape out of range");
+    if (shape[2] < 1 || double(shape[0]) * double(shape[1]) * double(shape[2]) >= double(1LL << 42))
+        return chg_fail(NDNLM_EINVAL, "needs at least 1 time step (and fewer than 2^42 samples)");
+    if (dtype != NDCHG_F32 && dtype != NDCHG_F64) return chg_fail(NDNLM_EDTYPE, "No matching signature found (only float32 / float64 data is supported)");
+    return NDNLM_OK;
+}
+
+template <typename T, int POL>
+static int run_zones(const void* values, const int64_t* shape, const int64_t* strides, int anisotropy, uint8_t* zones,
+                     cudaStream_t st) {
+    const long long rows = shape[0], cols = shape[1], k = shape[2], CH = ndchg::ZONE_CHUNK;
+    const long long samples = rows * cols * k;
+    T* scratch = nullptr;
+    cudaError_t e = cudaMallocAsync((void**)&scratch, sizeof(T) * size_t(samples < CH ? samples : CH) * ndchg::haa_outputs(POL), st);
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "scratch allocation failed: %s", cudaGetErrorString(e));
+    // one box of samples whose outputs are contiguous: rows r0.., or columns j0.. of row i, or steps t0.. of (i, j)
+    auto box = [&](long long i, long long j, long long t, long long nr, long long nc, long long nk) -> int {
+        const int64_t sub[3] = {nr, nc, nk};
+        const T* src = (const T*)values + i * strides[0] + j * strides[1] + t * strides[2];
+        int rc = launch_h_a_alpha<T, POL>(src, sub, strides, scratch, st);
+        if (rc) return rc;
+        const long long n = nr * nc * nk;
+        ndchg::h_alpha_zone_kernel<T, POL><<<unsigned((n + ndchg::HAA_THREADS - 1) / ndchg::HAA_THREADS), ndchg::HAA_THREADS, 0, st>>>(
+            scratch, n, anisotropy, zones + (i * cols + j) * k + t);
+        return NDNLM_OK;
+    };
+    int rc = NDNLM_OK;
+    if (cols * k <= CH) {
+        const long long rr = CH / (cols * k);
+        for (long long i = 0; i < rows && !rc; i += rr) rc = box(i, 0, 0, rows - i < rr ? rows - i : rr, cols, k);
+    } else if (k <= CH) {
+        const long long cc = CH / k;
+        for (long long i = 0; i < rows && !rc; ++i)
+            for (long long j = 0; j < cols && !rc; j += cc) rc = box(i, j, 0, 1, cols - j < cc ? cols - j : cc, k);
+    } else {
+        for (long long i = 0; i < rows && !rc; ++i)
+            for (long long j = 0; j < cols && !rc; ++j)
+                for (long long t = 0; t < k && !rc; t += CH) rc = box(i, j, t, 1, 1, k - t < CH ? k - t : CH);
+    }
+    cudaFreeAsync(scratch, st);
+    e = cudaGetLastError();
+    if (!rc && e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return rc;
+}
+
+template <typename T>
+static int run_zones(int pol, const void* values, const int64_t* shape, const int64_t* strides, int anisotropy, uint8_t* zones,
+                     cudaStream_t st) {
+    switch (pol) {
+        case NDCHG_POL_DUAL: return run_zones<T, NDCHG_POL_DUAL>(values, shape, strides, anisotropy, zones, st);
+        case NDCHG_POL_QUAD: return run_zones<T, NDCHG_POL_QUAD>(values, shape, strides, anisotropy, zones, st);
+        case NDCHG_POL_DUAL_DIAGONAL: return run_zones<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, anisotropy, zones, st);
+        case NDCHG_POL_QUAD_DIAGONAL: return run_zones<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, anisotropy, zones, st);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+extern "C" int ndchg_h_alpha_zones(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                                   int anisotropy, uint8_t* zones, void* stream) {
+    if (!values || !shape || !strides || !zones) return chg_fail(NDNLM_EINVAL, "null argument");
+    int rc = check_decomposable(pol);
+    if (rc) return rc;
+    if (anisotropy != 0 && anisotropy != 1) return chg_fail(NDNLM_EINVAL, "anisotropy must be 0 or 1, got %d", anisotropy);
+    if (anisotropy && pol != NDCHG_POL_QUAD && pol != NDCHG_POL_QUAD_DIAGONAL)
+        return chg_fail(NDNLM_EINVAL, "anisotropy needs a quad layout (the dual layouts have no A)");
+    rc = check_samples(shape, dtype);
+    if (rc) return rc;
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, zones, 1, 1))
+        return chg_fail(NDNLM_EINVAL, "zones must not overlap values");
+    ChgDeviceGuard guard(zones);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "zones is not a CUDA device pointer");
+    return dtype == NDCHG_F64 ? run_zones<double>(pol, values, shape, strides, anisotropy, zones, (cudaStream_t)stream)
+                              : run_zones<float>(pol, values, shape, strides, anisotropy, zones, (cudaStream_t)stream);
+}
+
+static bool is_device(const void* p) {
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, p) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return attr.type == cudaMemoryTypeDevice;
+}
+
+template <typename T, int POL>
+static int run_wishart(const void* values, const int64_t* shape, const int64_t* strides, uint8_t* labels, int K,
+                       uint32_t max_iter, double tol, double* centres, int64_t* counts, uint32_t* iterations, cudaStream_t st) {
+    using namespace ndchg;
+    constexpr int B = pol_bands(POL), E = B + 1;
+    const long long rows = shape[0], cols = shape[1], k = shape[2], samples = rows * cols * k;
+    const long long nchunk = (samples + WIS_CHUNK - 1) / WIS_CHUNK;
+    // (rows, cols, k) collapse into one axis of stride s2: sample g starts at element g * s2
+    const long long s1 = cols == 1 ? k * strides[2] : strides[1];
+    const bool flat = s1 == k * strides[2] && (rows == 1 || strides[0] == cols * s1);
+    const size_t state = (sizeof(WisState) + 255) / 256 * 256;
+    char* scratch = nullptr;
+    cudaError_t e = cudaMallocAsync((void**)&scratch, state + sizeof(double) * size_t(K * E) * (1 + nchunk), st);
+    if (e != cudaSuccess) return chg_fail(NDNLM_ECUDA, "scratch allocation of the Wishart sums failed: %s", cudaGetErrorString(e));
+    WisState* ws = (WisState*)scratch;
+    double* sums = (double*)(scratch + state);
+    double* partials = sums + K * E;
+    const size_t smem = wis_smem(POL, K);
+    e = cudaMemsetAsync(ws, 0, sizeof(WisState), st);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(wishart_assign_kernel<T, POL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(wishart_assign_kernel<T, POL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) {
+        cudaFreeAsync(scratch, st);
+        return chg_fail(NDNLM_ECUDA, "Wishart set-up failed: %s", cudaGetErrorString(e));
+    }
+    const long long check_blocks = (samples + 255) / 256;
+    wishart_check_kernel<<<unsigned(check_blocks < 4096 ? check_blocks : 4096), 256, 0, st>>>(labels, samples, K, ws);
+    auto pass = [&](unsigned it) {
+        if (it == 0)
+            wishart_assign_kernel<T, POL, false><<<unsigned(nchunk), WIS_THREADS, smem, st>>>(
+                (const T*)values, cols, k, samples, strides[0], strides[1], strides[2], strides[3], flat, labels, ws, K, partials, nchunk);
+        else
+            wishart_assign_kernel<T, POL, true><<<unsigned(nchunk), WIS_THREADS, smem, st>>>(
+                (const T*)values, cols, k, samples, strides[0], strides[1], strides[2], strides[3], flat, labels, ws, K, partials, nchunk);
+        wishart_reduce_kernel<<<unsigned(K * E), WIS_REDUCE_THREADS, 0, st>>>(partials, nchunk, sums, ws);
+        wishart_centres_kernel<POL><<<1, 32, 0, st>>>(ws, sums, K, it, max_iter, tol, centres, (long long*)counts, iterations);
+    };
+    // iteration 0, then one wait: a label > K or no active class is reported before any iteration is enqueued
+    pass(0);
+    unsigned status[3] = {0, 0, 0};                                      // done, bad, active
+    e = cudaMemcpyAsync(status, &ws->done, sizeof(status), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    int rc = NDNLM_OK;
+    if (e != cudaSuccess) rc = chg_fail(NDNLM_ECUDA, "iteration 0 failed: %s", cudaGetErrorString(e));
+    else if (status[1]) rc = chg_fail(NDNLM_EINVAL, "an initial label exceeds classes=%d", K);
+    else if (status[2] == 0)
+        rc = chg_fail(NDNLM_EINVAL, "no class is active after iteration 0 (every class is empty or its mean covariance is singular)");
+    // the iterations, in batches of 32: after each batch the host looks at the done flag once
+    for (uint32_t it = 1; !rc && !status[0] && it <= max_iter; ++it) {
+        pass(it);
+        if (it % 32 == 0 && it < max_iter) {
+            e = cudaMemcpyAsync(status, &ws->done, sizeof(unsigned), cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) rc = chg_fail(NDNLM_ECUDA, "iteration %u failed: %s", it, cudaGetErrorString(e));
+        }
+    }
+    cudaFreeAsync(scratch, st);
+    e = cudaGetLastError();
+    if (!rc && e != cudaSuccess) rc = chg_fail(NDNLM_ECUDA, "launch failed: %s", cudaGetErrorString(e));
+    return rc;
+}
+
+template <typename T>
+static int run_wishart(int pol, const void* values, const int64_t* shape, const int64_t* strides, uint8_t* labels, int K,
+                       uint32_t max_iter, double tol, double* centres, int64_t* counts, uint32_t* iterations, cudaStream_t st) {
+    switch (pol) {
+        case NDCHG_POL_DUAL:
+            return run_wishart<T, NDCHG_POL_DUAL>(values, shape, strides, labels, K, max_iter, tol, centres, counts, iterations, st);
+        case NDCHG_POL_QUAD:
+            return run_wishart<T, NDCHG_POL_QUAD>(values, shape, strides, labels, K, max_iter, tol, centres, counts, iterations, st);
+        case NDCHG_POL_DUAL_DIAGONAL:
+            return run_wishart<T, NDCHG_POL_DUAL_DIAGONAL>(values, shape, strides, labels, K, max_iter, tol, centres, counts, iterations, st);
+        case NDCHG_POL_QUAD_DIAGONAL:
+            return run_wishart<T, NDCHG_POL_QUAD_DIAGONAL>(values, shape, strides, labels, K, max_iter, tol, centres, counts, iterations, st);
+        default: return chg_fail(NDNLM_EINVAL, "unknown covariance layout pol=%d", pol);
+    }
+}
+
+extern "C" int ndchg_wishart_classify(const void* values, const int64_t shape[3], const int64_t strides[4], int dtype, int pol,
+                                      uint8_t* labels, uint32_t classes, uint32_t max_iter, double tol, double* centres,
+                                      int64_t* counts, uint32_t* iterations, void* stream) {
+    if (!values || !shape || !strides || !labels || !centres || !counts || !iterations) return chg_fail(NDNLM_EINVAL, "null argument");
+    int rc = check_decomposable(pol);
+    if (!rc) rc = check_samples(shape, dtype);
+    if (rc) return rc;
+    if (classes < 1 || classes > ndchg::WIS_MAX_CLASSES)
+        return chg_fail(NDNLM_EINVAL, "classes must be in [1, %d], got %u", ndchg::WIS_MAX_CLASSES, classes);
+    if (!(tol >= 0.0 && tol <= 1.0)) return chg_fail(NDNLM_EINVAL, "tol must be in [0, 1], got %g", tol);
+    if (lee_overlap(values, shape, strides, ndchg::pol_bands(pol), dtype == NDCHG_F64 ? 8 : 4, labels, 1, 1))
+        return chg_fail(NDNLM_EINVAL, "labels must not overlap values");
+    ChgDeviceGuard guard(labels);
+    if (!guard.ok) return chg_fail(NDNLM_EINVAL, "labels is not a CUDA device pointer");
+    if (!is_device(centres) || !is_device(counts) || !is_device(iterations))
+        return chg_fail(NDNLM_EINVAL, "centres, counts and iterations must be CUDA device pointers");
+    return dtype == NDCHG_F64 ? run_wishart<double>(pol, values, shape, strides, labels, int(classes), max_iter, tol, centres,
+                                                    counts, iterations, (cudaStream_t)stream)
+                              : run_wishart<float>(pol, values, shape, strides, labels, int(classes), max_iter, tol, centres,
+                                                   counts, iterations, (cudaStream_t)stream);
 }
 
 extern "C" const char* ndchg_last_error(void) { return g_chg_err; }
